@@ -7,6 +7,9 @@ h = 0.025, `odeint_adjoint` + `loss.backward()`.  A "step" of this bench is one 
 A trajectory-step = one sample advanced one accepted step forward plus its adjoint step (BASELINE.md section 3).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--dtype f64|f32] [--impl reference] [--no-configs]
+                    [--dump-outputs DIR]
+`--dump-outputs DIR` writes what the last timed pass handed its caller (see dump_outputs) as DIR/<name>.npy; the inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 Besides the headline the line carries `parity` (a 32-trajectory slice against the CPU oracle; at N > 1 bit-equality of mu
 across ranks) and `configs`: every BASELINE.json shape through the drop-in (bench_configs.py) -- ms per pass, rate, roofline,
 bounded CPU baseline at N = 1; the sharding configs (3, 4, 5) weak-scaled at N > 1.
@@ -54,7 +57,11 @@ def parse():
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config table (`configs` key of the JSON line)")
     ap.add_argument("--config-iters", type=int, default=5)
     ap.add_argument("--no-peer", action="store_true", help="N>1: all-reduce mu with NCCL instead of inside the adjoint kernel")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed pass to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def make_problem(ntraj, dtype, seed=0):
@@ -67,6 +74,24 @@ def make_problem(ntraj, dtype, seed=0):
     target = torch.randn(T_OUT, ntraj, 1, 2, generator=g, dtype=torch.float64).to(dtype)
     func = SpiralFunc(dtype=dtype)
     return func, u0, t, target
+
+
+DUMP_TRAJ = 1 << 17  # trajectories in the --dump-outputs sample of the solution: 21 MB in fp64
+
+
+def dump_outputs(path, pred, loss, func):
+    """What one pass hands its caller, in the run's dtype: `solution`, the trajectory at the output times
+    [T_OUT, n, 1, DIM] of a fixed seeded sample of n = min(batch, DUMP_TRAJ) trajectories in batch order; the scalar
+    `loss`; `grad_<parameter>` for every parameter of the model."""
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    ntraj = pred.shape[1]
+    idx = torch.randperm(ntraj, generator=torch.Generator().manual_seed(0))[:DUMP_TRAJ].sort().values
+    arrays = {"solution": pred.detach()[:, idx.to(pred.device)], "loss": loss.detach()}
+    arrays.update(("grad_" + name, p.grad) for name, p in func.named_parameters())
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a.cpu().numpy())
 
 
 def headline_config(world, ntraj, exchange):
@@ -127,18 +152,22 @@ def run_reference(args):
     ode = OracleODEPetsc(["-ts_adapt_type", "none", "-ts_trajectory_type", "memory"])
     ode.setupTS(u0, func, step_size=H, method="rk4", enable_adjoint=True)
 
-    def one():
+    def one(keep=False):
         func.zero_grad()
         pred = ode.odeint_adjoint(u0, t)
         loss = torch.mean(torch.abs(pred - target))
         loss.backward()
+        return (pred.detach(), loss.detach()) if keep else None
 
     for _ in range(max(args.warmup, 1)):
         one()
     t0 = time.perf_counter()
-    for _ in range(args.steps):
-        one()
+    for i in range(args.steps):
+        kept = one(keep=args.dump_outputs is not None and i == args.steps - 1)
     total = time.perf_counter() - t0
+    if kept is not None:
+        dump_outputs(args.dump_outputs, *kept, func)
+        del kept
     value = ntraj * NSTEPS * args.steps / total
     sample = "all %d trajectories of one GPU's batch per step (same model, schedule, dtype), %d warm-up + %d timed passes" % (
         ntraj, max(args.warmup, 1), args.steps)
@@ -321,11 +350,18 @@ def run_native(args):
             ode.comm.enable_peer_reduce()
     ode.setupTS(u0_dev, func, step_size=H, method="rk4", enable_adjoint=True)
 
+    # --dump-outputs: the pass numbered keep["at"] (the final timed one) keeps what it returned, detached so that its
+    # stage checkpoints are freed with the autograd graph; every other pass keeps nothing
+    keep = {"passes": 0, "at": None}
+
     def step_resident():
         func.zero_grad(set_to_none=True)
         pred = ode.odeint_adjoint(u0_dev, t_dev)
         loss = torch.mean(torch.abs(pred - target_dev))
         loss.backward()
+        keep["passes"] += 1
+        if keep["passes"] == keep["at"]:
+            keep["out"] = (pred.detach(), loss.detach())
         return loss
 
     grads_host = torch.empty(ode.np, dtype=dtype).pin_memory()
@@ -397,10 +433,14 @@ def run_native(args):
         assert parity["mu_bit_equal_across_ranks"], "mu differs between ranks after the all-reduce"
     fused = ode._fused
     l0 = fused.launches + ode._ops.launches
+    if args.dump_outputs and rank == 0:
+        keep["at"] = keep["passes"] + args.steps
     with ClockSampler(local) as clk:
         ms = timed(step_resident, args.steps)
     launches = fused.launches + ode._ops.launches - l0
     clocks = clk.summary()
+    if "out" in keep:  # before the passes below overwrite the gradients
+        dump_outputs(args.dump_outputs, *keep.pop("out"), func)
     total_units = world * ntraj * NSTEPS * args.steps
     value = total_units / (ms * 1e-3)
 
