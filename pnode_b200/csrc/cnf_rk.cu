@@ -24,24 +24,12 @@
 #include "common.cuh"
 #include "f32x2.cuh"
 
-// tuning switches (tools/tune_cnf.py builds -D variants; the defaults are the measured best)
-#ifndef CNF_PREFETCH
-#define CNF_PREFETCH 1   // adjoint: fetch a stage's checkpoint one stage ahead of its use
-#endif
-#ifndef CNF_F32ACC
-#define CNF_F32ACC 1     // adjoint, fp32: per-lane parameter-gradient sums in fp32 (fp64 from the block combine on)
-#endif
-#ifndef CNF_ACC_EARLY
-#define CNF_ACC_EARLY 1  // adjoint: read the chunk's accumulators before the phase-2 loop, not after it
-#endif
+// tuning parameters (tools/tune_cnf.py builds -D variants; the defaults are the measured best)
 #ifndef CNF_P1_UNROLL
 #define CNF_P1_UNROLL 2  // adjoint phase 1: hidden units in flight per thread
 #endif
 #ifndef CNF_P2_UNROLL
 #define CNF_P2_UNROLL 2  // adjoint phase 2: 16-byte trajectory vectors in flight per lane
-#endif
-#ifndef CNF_HOIST_Q
-#define CNF_HOIST_Q 1    // attempt kernel: q_j = W1[j,:] e once per attempt (a shared-memory column per thread), not per stage
 #endif
 #ifndef CNF_ATT_MINB
 #define CNF_ATT_MINB 2   // attempt kernel: CTAs per SM the register allocation aims at
@@ -193,7 +181,7 @@ __device__ __forceinline__ V sub_sum(V v) {
 // f(t_i, (z, .)): out[0..D) = dz, out[D] = -e^T J e -- for the Pack<T>::W trajectories a thread carries (fp64: one, plain
 // doubles; fp32: two, in the halves of packed registers, every operation an FFMA2 / FMUL2 / FADD2)
 // qcol: the thread's column of q_j = W1[j,:] e (stride CNF_THREADS), which does not depend on the stage -- computed once
-// per attempt by the caller; nullptr: recomputed here.
+// per attempt by the caller.
 template <typename T, int D, int H, int S, int LPT, typename V>
 __device__ __forceinline__ void cnf_eval(const CnfShared<T, D, H, S> &sm, int i, const V (&z)[D], const V (&e)[D],
                                          V (&out)[D + 1], const V *__restrict__ qcol, int qstride, int sub) {
@@ -209,14 +197,13 @@ __device__ __forceinline__ void cnf_eval(const CnfShared<T, D, H, S> &sm, int i,
     CNF_UNROLL(CNF_EVAL_UNROLL)
     for (int j = jbeg; j < jend; ++j) {
         const UnitC<T, D> u = sm.unit[j];
-        V p = Pack<T>::all(u.b1), q = Pack<T>::all(T(0)), w = Pack<T>::all(T(0));
+        V p = Pack<T>::all(u.b1), w = Pack<T>::all(T(0));
 #pragma unroll
         for (int k = 0; k < D; ++k) {
             p = fma(u.w1[k], z[k], p);
-            if (!CNF_HOIST_Q) q = fma(u.w1[k], e[k], q);
             w = fma(u.w2[k], ge[k], w);
         }
-        if (CNF_HOIST_Q) q = qcol[j * qstride];
+        const V q = qcol[j * qstride];
         const T g1 = sm.g1[i][j];
         const V a = fma(p, g1, sm.c1[i][j]);
         V s, sg;
@@ -412,14 +399,13 @@ cnf_rk_attempt_kernel(const CnfPtrs<T> w, const pnode_rk_tableau tab, const T *_
             e[k] = gather(w.e, D, k);
         }
         y[D] = gather(u, 1, ntraj * D);
-        if (CNF_HOIST_Q) {
+        // q_j = W1[j,:] e does not depend on the stage: once per attempt, into the thread's shared-memory column
 #pragma unroll 4
-            for (int j = sub * (H / LPT); j < (sub + 1) * (H / LPT); ++j) {
-                V q = P::all(T(0));
+        for (int j = sub * (H / LPT); j < (sub + 1) * (H / LPT); ++j) {
+            V q = P::all(T(0));
 #pragma unroll
-                for (int k = 0; k < D; ++k) q = fma(sm.unit[j].w1[k], e[k], q);
-                qcol[j * CNF_THREADS] = q;
-            }
+            for (int k = 0; k < D; ++k) q = fma(sm.unit[j].w1[k], e[k], q);
+            qcol[j * CNF_THREADS] = q;
         }
         if (sol_out != nullptr) {  // the state this attempt starts from landed on an output time
 #pragma unroll
@@ -636,12 +622,10 @@ template <typename T>
 struct AccType {
     typedef double type;
 };
-#if CNF_F32ACC
 template <>
 struct AccType<float> {
     typedef float type;
 };
-#endif
 
 template <typename T, int D, int H, int S, int LPT>
 __global__ void __launch_bounds__(CNF_ADJ_THREADS)
@@ -723,8 +707,7 @@ cnf_rk_adj_kernel(const CnfPtrs<T> w, const pnode_rk_tableau tab, const int64_t 
         V znext[D];
 #pragma unroll
         for (int k = 0; k < D; ++k)
-            znext[k] = CNF_PREFETCH ? gather(ckpt, 1, (((int64_t)(nsteps - 1) * s_eff + i_first) * D + k) * ntraj)
-                                    : P::all(T(0));
+            znext[k] = gather(ckpt, 1, (((int64_t)(nsteps - 1) * s_eff + i_first) * D + k) * ntraj);
 
         for (int n = nsteps - 1; n >= 0; --n) {
             const double h = sched[n].h;
@@ -757,15 +740,11 @@ cnf_rk_adj_kernel(const CnfPtrs<T> w, const pnode_rk_tableau tab, const int64_t 
                 V z[D], vg[D], ge[D], r[D], rho[D], dzk[D];
                 const T tt = sm.tstage[i];
 #pragma unroll
-                for (int k = 0; k < D; ++k)
-                    z[k] = CNF_PREFETCH ? znext[k] : gather(ckpt, 1, (((int64_t)n * s_eff + i) * D + k) * ntraj);
-                if (CNF_PREFETCH) {
-                    const int nn = i > 0 ? n : n - 1, in = i > 0 ? i - 1 : i_first;
-                    if (nn >= 0) {
+                for (int k = 0; k < D; ++k) z[k] = znext[k];
+                const int nn = i > 0 ? n : n - 1, in = i > 0 ? i - 1 : i_first;
+                if (nn >= 0) {
 #pragma unroll
-                        for (int k = 0; k < D; ++k)
-                            znext[k] = gather(ckpt, 1, (((int64_t)nn * s_eff + in) * D + k) * ntraj);
-                    }
+                    for (int k = 0; k < D; ++k) znext[k] = gather(ckpt, 1, (((int64_t)nn * s_eff + in) * D + k) * ntraj);
                 }
 #pragma unroll
                 for (int k = 0; k < D; ++k) {
@@ -823,7 +802,9 @@ cnf_rk_adj_kernel(const CnfPtrs<T> w, const pnode_rk_tableau tab, const int64_t 
                     __syncwarp();
                     // ---- phase 2 (lane = hidden unit x trajectory group): sums over the warp's trajectories -----------
                     if (pu < jn) {
-                        constexpr bool EARLY = CNF_ACC_EARLY && W == 2;  // fp64 has no registers to spare for it
+                        // the chunk's accumulators are read before the loop (fp32) so that their load hides behind it;
+                        // fp64 has no registers to spare for that and reads them after the loop
+                        constexpr bool EARLY = W == 2;
                         AccT ar[NA];
                         if (EARLY) {
 #pragma unroll
@@ -1032,7 +1013,7 @@ static int launch_cnf_attempt_lpt(const pnode_cnf_desc *c, const pnode_rk_tablea
                                   void *d_ubuf, void *d_kbuf, int64_t ckpt_step_elems, void *d_sol, int nlaunch,
                                   unsigned long long loop_cond, const PeerComm &pc) {
     auto kern = cnf_rk_attempt_kernel<T, 6, 60, S, LPT>;
-    const size_t smem = CNF_HOIST_Q ? sizeof(typename Pack<T>::V) * 60 * CNF_THREADS : 0;
+    const size_t smem = sizeof(typename Pack<T>::V) * 60 * CNF_THREADS;  // q_j columns
     static int ctas_per_sm = 0;
     if (ctas_per_sm == 0) {
         PNODE_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));

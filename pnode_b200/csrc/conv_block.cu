@@ -32,10 +32,8 @@
 // Measured dead ends (kept out of the code): a 64-register weight-gradient kernel so that it co-resides with the data-gradient
 // CTA (spills: 296 vs 287 us per adjoint stage); folding the producer warp into consumer warp 0 to fit two pipelined CTAs per SM
 // at 128 registers (warp 0 stalls on the slowest warp every chunk: 147 vs 107 us per evaluation on block 2).
-// Tuning knobs (environment, read once; the defaults are the measured best): PNODE_CONV_PIPE (0: direct-load kernels only),
-// PNODE_PIPE_RC / _STAGES / _CTAS / _SMEM_KB, PNODE_CONV_RC / _OCC (direct kernel), PNODE_WGRAD_OCC / _STREAM, PNODE_CONV_PDL.
+// The launch geometry (conv_grid, pipe_grid, cb_plan) is fixed at the measured best.
 #include <math.h>
-#include <stdlib.h>
 
 #include <map>
 
@@ -48,6 +46,7 @@
 #include "common.cuh"
 #include "f32x2.cuh"
 #include "graph_cache.cuh"
+#include "pdl.cuh"
 
 namespace pnode {
 
@@ -63,67 +62,26 @@ struct V4 {
     T v[4];
 };
 
-// acc[0..4) += w * o[0..4): four pixels of one output channel.  fp32: two packed FFMA2 (csrc/f32x2.cuh; the scalar weight is
-// broadcast by the instruction, the pixel pairs are adjacent registers of the 128-bit load they came from) -- half the issue
-// slots of four FFMA, identical rounding.
-#ifndef PNODE_CONV_FFMA2
-#define PNODE_CONV_FFMA2 1
-#endif
-// acc += sum_e a[e] b[e] over four pixels (weight-gradient tiles).  fp32: the accumulator is a packed pair holding the sums of
-// the even and the odd pixels (two FFMA2 instead of four dependent FFMA), added together once at the end.
-template <typename T>
-struct DotAcc {
-    typedef T type;
-};
-#ifndef PNODE_WGRAD_FFMA2
-#define PNODE_WGRAD_FFMA2 0  // measured on block 1 / 2: 1.59 -> 1.62 / 1.30 -> 1.33 ms per replayed pass, so off
-#endif
-#if PNODE_WGRAD_FFMA2
-template <>
-struct DotAcc<float> {
-    typedef F2 type;
-};
-__device__ __forceinline__ void dot4_acc(const V4<float> &a, const V4<float> &b, F2 &acc) {
-    acc = fma(pk(a.v[0], a.v[1]), pk(b.v[0], b.v[1]), acc);
-    acc = fma(pk(a.v[2], a.v[3]), pk(b.v[2], b.v[3]), acc);
-}
-__device__ __forceinline__ float dot_total(F2 acc) { return lo(acc) + hi(acc); }
-__device__ __forceinline__ void dot_zero(F2 &acc) { acc = splat(0.0f); }
-#endif
+// acc += sum_e a[e] b[e] over four pixels (weight-gradient tiles)
 template <typename T>
 __device__ __forceinline__ void dot4_acc(const V4<T> &a, const V4<T> &b, T &acc) {
 #pragma unroll
     for (int e = 0; e < 4; ++e) acc = fma(a.v[e], b.v[e], acc);
 }
-template <typename T>
-__device__ __forceinline__ T dot_total(T acc) {
-    return acc;
-}
-template <typename T>
-__device__ __forceinline__ void dot_zero(T &acc) {
-    acc = T(0);
-}
 
+// acc[0..4) += w * o[0..4): four pixels of one output channel.  fp32: two packed FFMA2 (csrc/f32x2.cuh; the scalar weight is
+// broadcast by the instruction, the pixel pairs are adjacent registers of the 128-bit load they came from) -- half the issue
+// slots of four FFMA, identical rounding.
 __device__ __forceinline__ void fma_row4(double w, const V4<double> &o, double (&acc)[4]) {
 #pragma unroll
     for (int j = 0; j < 4; ++j) acc[j] = fma(w, o.v[j], acc[j]);
 }
 __device__ __forceinline__ void fma_row4(float w, const V4<float> &o, float (&acc)[4]) {
-#if PNODE_CONV_FFMA2
     const F2 a = fma(w, pk(o.v[0], o.v[1]), pk(acc[0], acc[1]));
     const F2 b = fma(w, pk(o.v[2], o.v[3]), pk(acc[2], acc[3]));
     unpk(a, acc[0], acc[1]);
     unpk(b, acc[2], acc[3]);
-#else
-#pragma unroll
-    for (int j = 0; j < 4; ++j) acc[j] = fmaf(w, o.v[j], acc[j]);
-#endif
 }
-
-// Programmatic dependent launch: every kernel of this file lets its successor start early (its prologue -- barrier init, weight
-// staging -- overlaps this kernel's tail) and waits for its predecessor's memory before touching anything that depends on it.
-__device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
-__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 
 __device__ __forceinline__ V4<float> ld4(const float *p) {
     const float4 t = *reinterpret_cast<const float4 *>(p);
@@ -590,13 +548,13 @@ __global__ void __launch_bounds__(CB_PGX *CB_MAXCG) conv_kernel(const ConvArgs<T
     T *tout = tin + NCoef<SRC>::N * a.CA;     // [4][CT]   (EPI_DGRAD)
     const int cb0 = blockIdx.y * CT;
     const int tid = threadIdx.y * CB_PGX + threadIdx.x, nthr = CB_PGX * blockDim.y;
-    pdl_launch_dependents();
+    pdl::pdl_launch_dependents();
     for (int i = tid; i < a.CA * TAPS * CT; i += nthr) {
         const int bl = i % CT, ao = i / CT, o = ao % TAPS, ach = ao / TAPS, b = cb0 + bl;
         // forward: W[co = b][ci = ach][tap = o];  data gradient: W[co = ach][ci = b][tap = TAPS-1-o]
         ws[i] = FWD ? a.w[((int64_t)b * a.CA + ach) * TAPS + o] : a.w[((int64_t)ach * a.CB + b) * TAPS + (TAPS - 1 - o)];
     }
-    pdl_wait();
+    pdl::pdl_wait();
     fill_input_coefs<T, SRC>(tin, a.CA, a.bin, 0, a.CA, a.M, a.flag, tid, nthr);
     if constexpr (EPI == EPI_DGRAD) fill_output_coefs<T>(tout, CT, a.bout, cb0, CT, a.M, a.flag, tid, nthr);
     if (blockIdx.x == 0 && blockIdx.y == 0) {
@@ -736,10 +694,10 @@ __global__ void __launch_bounds__(CP_CONSUMERS + 32) convp_kernel(const ConvArgs
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    pdl_launch_dependents();
+    pdl::pdl_launch_dependents();
     __syncthreads();
     if (warp == CP_CONSUMERS / 32) {
-        pdl_wait();
+        pdl::pdl_wait();
         // ---- producer warp: every lane issues a share of the stage's bulk copies; lane 0 arms the barrier -------------------
         int slot = 0;
         uint32_t phase = 0;
@@ -780,7 +738,7 @@ __global__ void __launch_bounds__(CP_CONSUMERS + 32) convp_kernel(const ConvArgs
         const int bl = i % CT, ao = i / CT, o = ao % TAPS, ach = ao / TAPS, b = cb0 + bl;
         ws[i] = FWD ? a.w[((int64_t)b * a.CA + ach) * TAPS + o] : a.w[((int64_t)ach * a.CB + b) * TAPS + (TAPS - 1 - o)];
     }
-    pdl_wait();
+    pdl::pdl_wait();
     fill_input_coefs<T, SRC>(tin, a.CA, a.bin, 0, a.CA, a.M, a.flag, tid, CP_CONSUMERS);
     if constexpr (EPI == EPI_DGRAD) fill_output_coefs<T>(tout, CT, a.bout, cb0, CT, a.M, a.flag, tid, CP_CONSUMERS);
     if (blockIdx.x == 0 && blockIdx.y == 0) {
@@ -877,8 +835,8 @@ __global__ void __launch_bounds__(CB_PGX *CB_MAXCG) top_stats_kernel(const ConvA
     const int CT = blockDim.y * RC;
     const int cb0 = blockIdx.y * CT, ch0 = cb0 + threadIdx.y * RC;
     const int tid = threadIdx.y * CB_PGX + threadIdx.x, nthr = CB_PGX * blockDim.y;
-    pdl_launch_dependents();
-    pdl_wait();
+    pdl::pdl_launch_dependents();
+    pdl::pdl_wait();
     fill_output_coefs<T>(tout, CT, a.bout, cb0, CT, a.M, a.flag, tid, nthr);
     if (blockIdx.x == 0 && blockIdx.y == 0 && a.upd_out) bn_update_running<T>(a.bout, a.M, a.flag, tid, nthr);
     __syncthreads();
@@ -911,8 +869,8 @@ __global__ void __launch_bounds__(256) act_out_kernel(const T *__restrict__ z, c
     extern __shared__ __align__(128) unsigned char smem_raw[];
     T *tab = reinterpret_cast<T *>(smem_raw);  // [2][C]
     const int C = b.C;
-    pdl_launch_dependents();
-    pdl_wait();
+    pdl::pdl_launch_dependents();
+    pdl::pdl_wait();
     fill_input_coefs<T, SRC_ACT>(tab, C, b, 0, C, M, flag, threadIdx.x, blockDim.x);
     if (blockIdx.x == 0 && upd) bn_update_running<T>(b, M, flag, threadIdx.x, blockDim.x);
     __syncthreads();
@@ -975,19 +933,19 @@ __global__ void __launch_bounds__(WG_THREADS) conv_wgrad_kernel(const WgradArgs<
     const int ci_lo = cit0 / TAPS, ci_hi = min(a.Cin, (cit0 + WG_CIT - 1) / TAPS + 1);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int cgp = lane & 3, cg8 = lane >> 2;
-    pdl_launch_dependents();
+    pdl::pdl_launch_dependents();
     for (int i = threadIdx.x; i < (WG_CO + WG_CIT) * WG_LD; i += WG_THREADS) s_dz[i] = T(0);
-    pdl_wait();
+    pdl::pdl_wait();
     fill_input_coefs<T, SRC_DZ>(tdz, WG_CO, a.bk, co0, min(WG_CO, a.Cout - co0), a.M, a.flag, threadIdx.x, WG_THREADS);
     fill_input_coefs<T, YSRC>(ty, WG_CIT, a.bin, ci_lo, ci_hi - ci_lo, a.M, a.flag, threadIdx.x, WG_THREADS);
     __syncthreads();
     SD dsrc(a.g, a.z, tdz, WG_CO);
     SY ysrc(a.yin, nullptr, ty, WG_CIT);
-    typename DotAcc<T>::type acc[TM][TN];
+    T acc[TM][TN];
 #pragma unroll
     for (int i = 0; i < TM; ++i)
 #pragma unroll
-        for (int j = 0; j < TN; ++j) dot_zero(acc[i][j]);
+        for (int j = 0; j < TN; ++j) acc[i][j] = T(0);
     // this warp's rows of a chunk: NDZ dz rows (channels co0 + warp + 8 i) and NY source channels (ci_lo + warp + 8 u), clamped
     int rdz[NDZ], rci[NY];
 #pragma unroll
@@ -1052,7 +1010,7 @@ __global__ void __launch_bounds__(WG_THREADS) conv_wgrad_kernel(const WgradArgs<
 #pragma unroll
     for (int i = 0; i < TM; ++i)
 #pragma unroll
-        for (int j = 0; j < TN; ++j) red[warp * WG_TILE + (cgp + 4 * i) * WG_CIT + cg8 + 8 * j] = dot_total(acc[i][j]);
+        for (int j = 0; j < TN; ++j) red[warp * WG_TILE + (cgp + 4 * i) * WG_CIT + cg8 + 8 * j] = acc[i][j];
     __syncthreads();
     for (int idx = threadIdx.x; idx < WG_TILE; idx += WG_THREADS) {
         T t = T(0);
@@ -1085,8 +1043,8 @@ __global__ void __launch_bounds__(256) grads_finalize_kernel(const GradArgs<T> a
     const int sub = threadIdx.x % G;
     const int64_t stride = (int64_t)gridDim.x * (blockDim.x / G);
     const int64_t rounds = (a.np + stride - 1) / stride;
-    pdl_launch_dependents();
-    pdl_wait();
+    pdl::pdl_launch_dependents();
+    pdl::pdl_wait();
     const double bad = __ldcg(a.flag) != 0u ? NAN : 0.0;
     for (int64_t rd = 0; rd < rounds; ++rd) {
         const int64_t i = rd * stride + (int64_t)blockIdx.x * (blockDim.x / G) + threadIdx.x / G;
@@ -1149,16 +1107,12 @@ struct ConvGrid {
     size_t smem;
 };
 
-static int env_int(const char *name, int dflt) {
-    const char *v = getenv(name);
-    return v ? atoi(v) : dflt;
-}
-
-// One launcher for every kernel of this file: opt-in dynamic shared memory is raised once per kernel (not per launch), and the
-// launch carries the programmatic-stream-serialization attribute so that consecutive kernels overlap prologue and tail.
+// One launcher for every kernel of this file: opt-in dynamic shared memory is raised once per kernel (not per launch), then
+// pdl::launch_pdl launches it as a programmatic dependent launch.  Every kernel of this file lets its successor start early
+// (its prologue -- barrier init, weight staging -- overlaps this kernel's tail) and waits for its predecessor's memory before
+// touching anything that depends on it.
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args... args) {
-    static const int pdl = env_int("PNODE_CONV_PDL", 1);
     static std::map<const void *, size_t> raised;
     if (smem > 48 * 1024 - 4096) {
         size_t &have = raised[reinterpret_cast<const void *>(kernel)];
@@ -1168,25 +1122,15 @@ static cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, siz
             have = smem;
         }
     }
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr, cfg.numAttrs = pdl ? 1 : 0;
-    return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+    return pdl::launch_pdl(kernel, grid, block, smem, st, args...);
 }
 
 // thread = 4 pixels x rc output channels, CTA = 64 pixel groups x cg channel groups, grid.y = further channel tiles
 static ConvGrid conv_grid(int CA, int CB, int taps, int ncoef_in, bool dgrad_epi, int64_t npg, size_t esz) {
     ConvGrid g;
     const int sm = sm_count();
-    static const int want_rc = env_int("PNODE_CONV_RC", 8);  // tuning knobs
-    static const int occ = env_int("PNODE_CONV_OCC", 1024);
-    g.rc = want_rc;
-    if (g.rc == 16 && (CB % 16 != 0 || esz == 8)) g.rc = 8;
-    if (g.rc == 8 && CB % 8 != 0) g.rc = 4;
-    if (g.rc != 4 && g.rc != 8 && g.rc != 16) g.rc = 4;
+    constexpr int occ = 1024;  // resident threads per SM the grid aims at
+    g.rc = CB % 8 == 0 ? 8 : 4;
     int groups = CB / g.rc;
     g.cg = groups < CB_MAXCG ? groups : CB_MAXCG;
     while (groups % g.cg != 0) --g.cg;
@@ -1279,7 +1223,7 @@ static int cb_plan(const pnode_convblock_desc *d, CbPlan &p) {
         p.wg_tiles_cit[k] = (l.cin * p.taps[k] + wg_cit - 1) / wg_cit;
         p.wg_ntiles[k] = ((l.cout + wg_co - 1) / wg_co) * p.wg_tiles_cit[k];
         const int nchunks = (int)((p.npg + 31) / 32);
-        static const int wg_occ = env_int("PNODE_WGRAD_OCC", 2);  // 2: measured best with the side stream (271 vs 289 us at 4)
+        constexpr int wg_occ = 2;  // CTAs per SM: measured best with the side stream (271 vs 289 us at 4)
         int px = sm * wg_occ / p.wg_ntiles[k];
         if (px < 1) px = 1;
         if (px > nchunks) px = nchunks;
@@ -1302,12 +1246,9 @@ struct PipeGrid {
 // geometry of the pipelined kernel, or ok = false when the shape needs the direct kernel (halo rows, odd channel counts)
 static PipeGrid pipe_grid(int kind, int src, int CA, int CB, int taps, int64_t npg, int HW, size_t esz) {
     PipeGrid g = {};
-    static const int enabled = env_int("PNODE_CONV_PIPE", 1);
-    static const int want_rc = env_int("PNODE_PIPE_RC", 16);
-    static const int want_s = env_int("PNODE_PIPE_STAGES", 4);
-    static const int ctas_per_sm = env_int("PNODE_PIPE_CTAS", 2);
-    if (!enabled) return g;
-    const int rcmax = esz == 8 ? 8 : (want_rc >= 16 ? 16 : 8);
+    constexpr int max_stages = 4, ctas_per_sm = 2;
+    constexpr size_t smem_cap = 110 * 1024;  // per CTA, so that ctas_per_sm fit on an SM: stages are dropped (down to 2) first
+    const int rcmax = esz == 8 ? 8 : 16;
     g.rc = 0;
     for (int rc = rcmax; rc >= (esz == 8 ? 4 : 8); rc >>= 1)
         if (CB % rc == 0) {
@@ -1326,9 +1267,8 @@ static PipeGrid pipe_grid(int kind, int src, int CA, int CB, int taps, int64_t n
     const int CT = g.cg * g.rc;
     const size_t head = (128 + ((size_t)CA * taps * CT + (size_t)ncoef * CA + 4 * CT) * esz + 127) & ~(size_t)127;
     const size_t stage = (size_t)NT * KC * TP * esz;
-    g.S = want_s < 2 ? 2 : (want_s > 8 ? 8 : want_s);
-    static const int smem_cap = env_int("PNODE_PIPE_SMEM_KB", 110);
-    while (g.S > 2 && head + g.S * stage > (size_t)smem_cap * 1024) --g.S;
+    g.S = max_stages;
+    while (g.S > 2 && head + g.S * stage > smem_cap) --g.S;
     g.smem = head + g.S * stage;
     if (g.smem > 200 * 1024) return g;
     g.tiles = (int)((npg + PGT - 1) / PGT);
@@ -1360,15 +1300,8 @@ static int launch_conv_rc(const ConvArgs<T> &a_in, const ConvGrid &g, cudaStream
     }
     const ConvArgs<T> &a = a_in;
     dim3 grid(g.gx, g.gy), block(CB_PGX, g.cg);
-#define PNODE_CONV_LAUNCH(RC) PNODE_CUDA_OK(launch_k(conv_kernel<T, KIND, SRC, EPI, RC>, grid, block, g.smem, st, a))
-    if (g.rc == 16) {
-        if constexpr (sizeof(T) == 4) PNODE_CONV_LAUNCH(16);
-    } else if (g.rc == 8) {
-        PNODE_CONV_LAUNCH(8);
-    } else {
-        PNODE_CONV_LAUNCH(4);
-    }
-#undef PNODE_CONV_LAUNCH
+    if (g.rc == 8) PNODE_CUDA_OK(launch_k(conv_kernel<T, KIND, SRC, EPI, 8>, grid, block, g.smem, st, a));
+    else PNODE_CUDA_OK(launch_k(conv_kernel<T, KIND, SRC, EPI, 4>, grid, block, g.smem, st, a));
     return 0;
 }
 
@@ -1415,8 +1348,7 @@ static SideStream &side_stream() {
     static bool tried = false;
     if (!tried) {
         tried = true;
-        static const int enabled = env_int("PNODE_WGRAD_STREAM", 1);
-        bool ok = enabled && cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) == cudaSuccess;
+        bool ok = cudaStreamCreateWithFlags(&s.stream, cudaStreamNonBlocking) == cudaSuccess;
         for (int i = 0; ok && i <= PNODE_CONV_MAX_LAYERS; ++i) ok = cudaEventCreateWithFlags(&s.fork[i], cudaEventDisableTiming) == cudaSuccess;
         ok = ok && cudaEventCreateWithFlags(&s.join, cudaEventDisableTiming) == cudaSuccess;
         s.ok = ok;
@@ -1518,13 +1450,8 @@ static int vjp_chain(const pnode_convblock_desc *d, const CbPlan &p, const Bufs<
         const ConvGrid g = conv_grid(0, l.cout, 1, 0, true, p.npg, p.esz);
         dim3 grid(g.gx, g.gy), block(CB_PGX, g.cg);
         const size_t smem = (size_t)4 * g.cg * g.rc * sizeof(T);
-        if (g.rc == 16) {
-            if constexpr (sizeof(T) == 4) PNODE_CUDA_OK(launch_k(top_stats_kernel<T, 16>, grid, block, smem, st, a));
-        } else if (g.rc == 8) {
-            PNODE_CUDA_OK(launch_k(top_stats_kernel<T, 8>, grid, block, smem, st, a));
-        } else {
-            PNODE_CUDA_OK(launch_k(top_stats_kernel<T, 4>, grid, block, smem, st, a));
-        }
+        if (g.rc == 8) PNODE_CUDA_OK(launch_k(top_stats_kernel<T, 8>, grid, block, smem, st, a));
+        else PNODE_CUDA_OK(launch_k(top_stats_kernel<T, 4>, grid, block, smem, st, a));
     }
     const T *gk = w;
     SideStream &side = side_stream();

@@ -17,9 +17,6 @@ VARIANTS = {
     "ev4_mb3": {"CNF_EVAL_UNROLL": 4, "CNF_ATT_MINB": 3},
     "ev2_mb3": {"CNF_EVAL_UNROLL": 2, "CNF_ATT_MINB": 3},
     "ev6": {"CNF_EVAL_UNROLL": 6},
-    "ev4_nohoist": {"CNF_EVAL_UNROLL": 4, "CNF_HOIST_Q": 0},
-    "ev4_nohoist_mb3": {"CNF_EVAL_UNROLL": 4, "CNF_HOIST_Q": 0, "CNF_ATT_MINB": 3},
-    "ev2_nohoist_mb4": {"CNF_EVAL_UNROLL": 2, "CNF_HOIST_Q": 0, "CNF_ATT_MINB": 4},
 }
 
 

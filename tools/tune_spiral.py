@@ -15,13 +15,9 @@ TUNE = os.path.join(CSRC, "tune")
 VARIANTS = {
     "base": {},
     "f64_tanh_v0": {"PNODE_F64_TANH_V": 0},       # relative-accuracy tanh (15 FP64 instructions)
-    "f64_park_s": {"PNODE_ADJ_RECOMPUTE_S": 0},   # adjoint phase 2 reads a parked copy of s
     "f32_t1c2": {"PNODE_F32_TPT": 1, "PNODE_F32_CHUNKS": 2, "PNODE_F32_ADJ_CTAS": 5},
     "f32_t1c2_ag1": {"PNODE_F32_TPT": 1, "PNODE_F32_CHUNKS": 2, "PNODE_F32_ADJ_CTAS": 5, "PNODE_F32_ADJ_GROUP": 1},
     "f32_t1c2_ag2": {"PNODE_F32_TPT": 1, "PNODE_F32_CHUNKS": 2, "PNODE_F32_ADJ_CTAS": 5, "PNODE_F32_ADJ_GROUP": 2},
-    "f32_t1c2_unroll": {"PNODE_F32_TPT": 1, "PNODE_F32_CHUNKS": 2, "PNODE_F32_ADJ_CTAS": 5, "PNODE_ADJ_ROLL": 0},
-    "f32_t1c2_ag1_unroll": {"PNODE_F32_TPT": 1, "PNODE_F32_CHUNKS": 2, "PNODE_F32_ADJ_CTAS": 5, "PNODE_F32_ADJ_GROUP": 1,
-                            "PNODE_ADJ_ROLL": 0},
     "f32_t2c2": {"PNODE_F32_CHUNKS": 2, "PNODE_F32_ADJ_CTAS": 3},
     "f32_t2c3_a3": {"PNODE_F32_ADJ_CTAS": 3},
     "f32_t2c3_ag1": {"PNODE_F32_ADJ_GROUP": 1, "PNODE_F32_ADJ_CTAS": 3},
@@ -29,7 +25,6 @@ VARIANTS = {
     "f32_fwd_t1": {"PNODE_F32_TPT": 1, "PNODE_F32_CHUNKS": 2, "PNODE_F32_ADJ_CTAS": 5, "PNODE_F32_FWD_CTAS": 12},
     "f64_ag10": {"PNODE_F64_ADJ_GROUP": 10},
     "f64_adj2": {"PNODE_F64_ADJ_CTAS": 2},
-    "f64_unroll": {"PNODE_ADJ_ROLL": 0},
     "f64_fwd4": {"PNODE_F64_FWD_CTAS": 4},
     "f64_fwd6": {"PNODE_F64_FWD_CTAS": 6},
     "f64_g10": {"PNODE_F64_GROUP": 10, "PNODE_F64_ADJ_GROUP": 5, "PNODE_F64_FWD_CTAS": 4},
