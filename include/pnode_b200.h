@@ -435,10 +435,13 @@ int pnode_cnf_rk_adjoint_dp(const pnode_cnf_desc *cnf, const pnode_rk_tableau *t
  * up to 128 bytes) such that products of slices are exact on the tensor cores:
  *   PNODE_SLICED_I8   fp64 source: x[r][c] = 2^exp[r] * sum_s q_s[r][c] 2^-(6+8s), q_s signed bytes (balanced base-256
  *                     digits), S = PNODE_I8_SLICES = 6 (Ozaki splitting: int8 x int8 -> int32 products are exact on the
- *                     tensor cores; 46 bits of every entry relative to its row maximum, rounded to nearest, are kept; a
- *                     product needs the 21 slice pairs i + j < 6).  Reduction length <= PNODE_I8_MAX_K (int32 accumulators).
- *   PNODE_SLICED_I8X  signed digits in [-64, 64], base 128, S = PNODE_I8X_SLICES = 8 (55 bits, 36 slice pairs, any reduction
- *                     length <= 65536): the truncation error of a sliced product is relative to (row maximum)(column
+ *                     tensor cores; 46 bits of every entry relative to its row maximum, rounded to nearest, are kept for
+ *                     row maxima in [2^-961, 2^960); the row exponent is clamped to [-960, 960], so smaller rows keep 46
+ *                     bits relative to 2^-960 and rows of 2^960 and above are outside the range; a product needs the 21
+ *                     slice pairs i + j < 6).  Reduction length <= PNODE_I8_MAX_K (int32 accumulators).
+ *   PNODE_SLICED_I8X  signed digits in [-64, 64], base 128, S = PNODE_I8X_SLICES = 8 (55 bits, same exponent range, 36 slice
+ *                     pairs, reduction length <= PNODE_I8X_MAX_K = 65535: diagonal 7 sums 8 digit pairs of up to 64 x 64 per
+ *                     reduction index in int32): the truncation error of a sliced product is relative to (row maximum)(column
  *                     maximum), so products whose terms cancel by many orders of magnitude -- applying (shift I - J)^-1 of a
  *                     stiff operator to a rough vector -- need the extra digits to stay at fp64 level
  *   PNODE_SLICED_TF32 fp32 source: x = hi + lo with hi = tf32(x), S = 2 (3xTF32: hi.hi + hi.lo + lo.hi)
@@ -455,6 +458,7 @@ int pnode_cnf_rk_adjoint_dp(const pnode_cnf_desc *cnf, const pnode_rk_tableau *t
 #define PNODE_I8_SLICES 6
 #define PNODE_I8X_SLICES 8
 #define PNODE_I8_MAX_K 16384
+#define PNODE_I8X_MAX_K 65535
 int64_t pnode_sliced_bytes(int kind, int rows, int k);
 int pnode_slice_rows(int kind, const void *d_x, int64_t ldx, int rows, int k, void *d_slices, int32_t *d_exp, void *stream);
 int pnode_slice_cols(int kind, const void *d_x, int64_t ldx, int rows, int cols, void *d_slices, int32_t *d_exp,

@@ -45,13 +45,16 @@ static int make_layout(const pnode_dmlp_desc *d, Layout &lay) {
     }
     lay.esz = d->dtype == PNODE_F64 ? 8 : 4;
     lay.batch = d->batch;
+    // every width and the batch are the reduction length of some product; fp64 beyond 16384 uses the 8-digit kind
+    const int max_k = d->dtype == PNODE_F64 ? PNODE_I8X_MAX_K : 65536;
     int maxdim = 0;
     for (int l = 0; l <= lay.L; ++l) {
-        PNODE_REQUIRE(d->dims[l] >= 1 && d->dims[l] <= 65536, "dense mlp: layer width %d", d->dims[l]);
+        PNODE_REQUIRE(d->dims[l] >= 1 && d->dims[l] <= max_k, "dense mlp: layer width %d (max %d)", d->dims[l], max_k);
         lay.dims[l] = d->dims[l];
         maxdim = d->dims[l] > maxdim ? d->dims[l] : maxdim;
     }
-    PNODE_REQUIRE(d->batch <= 65536, "dense mlp: batch %d exceeds the reduction length of one product", d->batch);
+    PNODE_REQUIRE(d->batch <= max_k, "dense mlp: batch %d exceeds the reduction length of one product (max %d)", d->batch,
+                  max_k);
     long long off = 0;
     for (int l = 0; l < lay.L; ++l) {
         const int in = lay.dims[l], out = lay.dims[l + 1];

@@ -5,11 +5,14 @@
 // reference to 1e-10 / 1e-4.  The 5th-generation tensor cores have no fp64 mode and TF32 alone is 1e-3, so every
 // operand is a SLICED matrix and a product is a short sum of exact slice products:
 //
-//   kind i8   (fp64):  x[r][k] = 2^e[r] * sum_s q_s[r][k] 2^-(6+7s),  q_s int8 in [-64, 64], S = 7 slices (48 bits).
-//              A.B^T = 2^(ea+eb) * sum_{d<S} 2^-(12+7d) * sum_{i+j=d} (q^A_i . q^B_j)      [Ozaki splitting]
+//   kind i8   (fp64):  x[r][k] = 2^e[r] * sum_s q_s[r][k] 2^-(6+8s),  q_s signed bytes (balanced base-256 digits),
+//              S = 6 slices (46 bits).
+//              A.B^T = 2^(ea+eb) * sum_{d<S} 2^-(12+8d) * sum_{i+j=d} (q^A_i . q^B_j)      [Ozaki splitting]
 //              every slice product is an EXACT int32 dot product (tcgen05.mma kind::i8), one TMEM accumulator per
-//              diagonal d; the fp64 combination happens once, in the epilogue.  Dropped terms are < 2^-47 of
-//              (row max)(column max) per term.
+//              diagonal d; the fp64 combination happens once, in the epilogue.  A diagonal sums up to 6 pairs of
+//              digits per reduction index, so the int32 accumulators (which wrap: no saturation) bound K <= 16384.
+//   kind i8x  (fp64):  8 signed base-128 digits in [-64, 64] (55 bits); diagonal 7 reaches 8 * 64 * 64 * K, which
+//              fits int32 up to K = 65535.
 //   kind tf32 (fp32):  x = hi + lo, hi = tf32(x), lo = x - hi;  A.B^T = hi.hi + hi.lo + lo.hi  (3xTF32, fp32 accumulate
 //              in TMEM), relative error ~2^-21 per product.
 //
@@ -38,7 +41,7 @@ struct Cfg<KIND_I8> {  // dense digits: base 256, balanced (all signed bytes) ->
 template <>
 struct Cfg<KIND_I8X> {  // one more slice (55 bits): products with heavy cancellation (stiff inverse apply)
     static constexpr int S = PNODE_I8X_SLICES, BN = 64, KB = 64, STAGES = 2, NACC = PNODE_I8X_SLICES, ELEM = 1;
-    static constexpr bool INT = true, DENSE = false;  // signed digits in [-64, 64] (base 128): any reduction length
+    static constexpr bool INT = true, DENSE = false;  // signed digits in [-64, 64] (base 128): K <= PNODE_I8X_MAX_K
     static constexpr int BASE_BITS = 7, LEAD_BITS = 6;
     using Out = double;
 };
@@ -799,6 +802,9 @@ int gemm_ex(int kind, const void *a, const void *b, int M, int N, int K, const E
     // dense digits: a diagonal accumulates up to S products of 255 x 255 per reduction index in int32
     PNODE_REQUIRE(kind != KIND_I8 || K <= PNODE_I8_MAX_K, "umma gemm: reduction length %d exceeds %d for PNODE_SLICED_I8 "
                   "(use PNODE_SLICED_I8X)", K, PNODE_I8_MAX_K);
+    // 8 digit pairs of up to 64 x 64 per reduction index on diagonal 7: 2^31 at K = 65536, one past INT32_MAX
+    PNODE_REQUIRE(kind != KIND_I8X || K <= PNODE_I8X_MAX_K, "umma gemm: reduction length %d exceeds %d for PNODE_SLICED_I8X",
+                  K, PNODE_I8X_MAX_K);
     if (kind == KIND_I8) return launch_gemm<KIND_I8>(a, b, M, N, K, ep, stream);
     if (kind == KIND_I8X) return launch_gemm<KIND_I8X>(a, b, M, N, K, ep, stream);
     if (kind == KIND_TF32) return launch_gemm<KIND_TF32>(a, b, M, N, K, ep, stream);
