@@ -221,8 +221,9 @@ def cfg2(dtype="f32", ntraj=1 << 20, lean=False):
 
 def _cnf(B, dtype, D=6, hidden=(60,), fixed_rk4=None):
     """FFJORD tabular CNF.  Default: the POWER shape of BASELINE config 3 (fused kernels, dopri5 adaptive).  Other shapes --
-    e.g. the reference's own usage line, train_tabular.py:5: miniboone, D=43, two hidden layers of 860, RK4 h=0.25 -- are
-    outside the fused recognisers and show what the generic stage loop does with them."""
+    e.g. the reference's own usage line, train_tabular.py:5: miniboone, D=43, two hidden layers of 860, RK4 h=0.25 -- run
+    the generic stage loop with the tensor-core evaluator of csrc/cnf_net.cu; the same call also times the module path
+    (-pnode_fused 0) for comparison."""
     from _workloads import CNFFunc, cnf_to
 
     def build():
@@ -245,8 +246,9 @@ def _cnf(B, dtype, D=6, hidden=(60,), fixed_rk4=None):
         if fixed_rk4 is not None:
             dims = (D,) + tuple(hidden) + (D,)
             f_f = 2 * 2 * sum(a * b for a, b in zip(dims[:-1], dims[1:]))  # network + Hutchinson VJP
-            return dict(desc="FFJORD tabular CNF D=%d hidden %s, B=%d, RK4 h=%g, t=[0,1], Hutchinson trace, %s (outside the "
-                             "fused recognisers)" % (D, "x".join(map(str, hidden)), B, fixed_rk4, dtype), dtype=dtype,
+            return dict(desc="FFJORD tabular CNF D=%d hidden %s, B=%d, RK4 h=%g, t=[0,1], Hutchinson trace, %s (ConcatSquash "
+                             "network evaluator, csrc/cnf_net.cu)" % (D, "x".join(map(str, hidden)), B, fixed_rk4, dtype),
+                        dtype=dtype, also_generic=True,
                         argv=["-ts_adapt_type", "none", "-ts_trajectory_type", "memory"], funcs=[full["func"]], u0=full["u0"],
                         t=t, target=full["target"], kw=dict(method="rk4"), step=fixed_rk4, batch=B, flops_per_unit=16 * f_f,
                         bytes_per_unit=(2 * 4 + 2) * (D + 1) * (4 if dtype == "f32" else 8),

@@ -508,6 +508,42 @@ int pnode_dmlp_vjp(const pnode_dmlp_desc *desc, const void *d_wslices, const voi
 int pnode_dmlp_vjp_ev(const pnode_dmlp_desc *desc, const void *d_wslices, const void *d_act, const void *d_w, void *d_vu,
                       void *d_mu, double coef, void *d_work, void *const *layer_events, void *stream);
 
+/* ----------------------------------------------------------------------------------------------------------------
+ * FFJORD right-hand side with an ODEnet of any depth (csrc/cnf_net.cu): L ConcatSquashLinear layers with Softplus(beta=1,
+ * threshold=20) between them, Hutchinson trace with the probe d_e, state cat(z.view(-1), logp.view(-1)) of B samples.
+ * Replaces ODEfunc.forward (ffjord-pnode/lib/layers/odefunc.py:53-57, 345-385; ConcatSquashLinear, diffeq_layers/basic.py:
+ * 76-86) in evalRHSFunction, and the second-order autograd of RHSJacShell.multTranspose + RHSJacPShell.multTranspose
+ * (pnode/petsc_adjoint.py:52-82, 341-363) in every adjoint stage.  Every product runs on the tensor cores through the
+ * sliced operands above (fp64: int8 slices, I8X when 2B or a width exceeds PNODE_I8_MAX_K; fp32: 3xTF32), with the value
+ * and tangent chains stacked as 2B rows.
+ *   prepare : slice every weight matrix in both orientations (once per solve: parameters are borrowed)
+ *   forward : d_out[B*(D+1)] = F(t, d_u); with d_act != NULL the evaluation keeps what the adjoint stage at the same point
+ *             needs (column-sliced layer inputs, pre-activations, gates)
+ *   vjp     : from the activation set of a forward at the same t: d_vu = J^T w (skipped if NULL); if d_mu != NULL,
+ *             mu[<param>_off[l] ...] += coef * d<param>_l (offsets in elements, -1: that parameter takes no gradient).
+ *             Bit-reproducible: the column sums are combined in a fixed order.
+ * -------------------------------------------------------------------------------------------------------------- */
+typedef struct pnode_cnfnet_desc {
+    int32_t nlayers, dtype, batch, t_f32;         /* t_f32 = 1: the module rounds t through float32 (odefunc.py:356) */
+    int32_t dims[PNODE_DMLP_MAX_LAYERS + 1];      /* dims[0] = D ... dims[nlayers] = D */
+    const void *d_weight[PNODE_DMLP_MAX_LAYERS];  /* _layer.weight [dims[l+1]][dims[l]] */
+    const void *d_bias[PNODE_DMLP_MAX_LAYERS];    /* _layer.bias [dims[l+1]] */
+    const void *d_hyper_bias[PNODE_DMLP_MAX_LAYERS];  /* _hyper_bias.weight [dims[l+1]][1] */
+    const void *d_gate_weight[PNODE_DMLP_MAX_LAYERS]; /* _hyper_gate.weight [dims[l+1]][1] */
+    const void *d_gate_bias[PNODE_DMLP_MAX_LAYERS];   /* _hyper_gate.bias [dims[l+1]] */
+    int64_t mu_w_off[PNODE_DMLP_MAX_LAYERS], mu_b_off[PNODE_DMLP_MAX_LAYERS], mu_hbw_off[PNODE_DMLP_MAX_LAYERS],
+        mu_hgw_off[PNODE_DMLP_MAX_LAYERS], mu_hgb_off[PNODE_DMLP_MAX_LAYERS];
+    const void *d_e;                              /* [B][D] Hutchinson probe */
+} pnode_cnfnet_desc;
+int64_t pnode_cnfnet_weight_bytes(const pnode_cnfnet_desc *desc);   /* -1: unsupported (pnode_last_error) */
+int64_t pnode_cnfnet_act_bytes(const pnode_cnfnet_desc *desc);
+int64_t pnode_cnfnet_work_bytes(const pnode_cnfnet_desc *desc);
+int pnode_cnfnet_prepare(const pnode_cnfnet_desc *desc, void *d_wslices, void *stream);
+int pnode_cnfnet_forward(const pnode_cnfnet_desc *desc, const void *d_wslices, double t, const void *d_u, void *d_out,
+                         void *d_act, void *d_work, void *stream);
+int pnode_cnfnet_vjp(const pnode_cnfnet_desc *desc, const void *d_wslices, double t, const void *d_act, const void *d_w,
+                     void *d_vu, void *d_mu, double coef, void *d_work, void *stream);
+
 /* Circulant linear operator J[i][j] = c[(i - j) mod n] applied to every row of d_x[rows][n] (the implicit half of the
  * SINODE pair: a circular-padding Conv1d stencil, imex.py:6-44; replaces evalIFunction's func(t, u), petsc_adjoint.py:
  * 414-431, and IJacShell's J^T x, 179-196).  `offsets` / `coefs` (HOST arrays, ntaps <= PNODE_CIRC_MAX_TAPS) list the

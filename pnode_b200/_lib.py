@@ -62,6 +62,14 @@ class DmlpDesc(C.Structure):
                 ("mu_b_off", C.c_int64 * DMLP_MAX_LAYERS), ("out_scale", C.c_double)]
 
 
+class CnfNetDesc(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("nlayers", "dtype", "batch", "t_f32")] + \
+               [("dims", C.c_int32 * (DMLP_MAX_LAYERS + 1))] + \
+               [(n, C.c_void_p * DMLP_MAX_LAYERS) for n in ("d_weight", "d_bias", "d_hyper_bias", "d_gate_weight",
+                                                            "d_gate_bias")] + \
+               [(n, C.c_int64 * DMLP_MAX_LAYERS) for n in ("mu_w_off", "mu_b_off", "mu_hbw_off", "mu_hgw_off",
+                                                          "mu_hgb_off")] + [("d_e", C.c_void_p)]
+
 
 class ConvLayer(C.Structure):
     _fields_ = [(n, C.c_int32) for n in ("cin", "cout", "kh", "kw", "ph", "pw")] + \
@@ -146,7 +154,13 @@ _SIGNATURES = {
     "pnode_dmlp_forward": (C.c_int, [C.POINTER(DmlpDesc), _vp, _vp, _vp, _vp, _vp, _vp]),
     "pnode_dmlp_vjp": (C.c_int, [C.POINTER(DmlpDesc), _vp, _vp, _vp, _vp, _vp, _d, _vp, _vp]),
     "pnode_dmlp_vjp_ev": (C.c_int, [C.POINTER(DmlpDesc), _vp, _vp, _vp, _vp, _vp, _d, _vp, _vp, _vp]),
-    "pnode_circulant_apply": (C.c_int, [_vp, _vp, _i, _i, C.POINTER(C.c_int32), C.POINTER(_d), _i, _i, _i, _vp]),
+    "pnode_cnfnet_weight_bytes": (_i64, [C.POINTER(CnfNetDesc)]),
+    "pnode_cnfnet_act_bytes": (_i64, [C.POINTER(CnfNetDesc)]),
+    "pnode_cnfnet_work_bytes": (_i64, [C.POINTER(CnfNetDesc)]),
+    "pnode_cnfnet_prepare": (C.c_int, [C.POINTER(CnfNetDesc), _vp, _vp]),
+    "pnode_cnfnet_forward": (C.c_int, [C.POINTER(CnfNetDesc), _vp, _d, _vp, _vp, _vp, _vp, _vp]),
+    "pnode_cnfnet_vjp": (C.c_int, [C.POINTER(CnfNetDesc), _vp, _d, _vp, _vp, _vp, _vp, _d, _vp, _vp]),
+    "pnode_circulant_apply":(C.c_int, [_vp, _vp, _i, _i, C.POINTER(C.c_int32), C.POINTER(_d), _i, _i, _i, _vp]),
     "pnode_circulant_work_bytes": (_i64, [_i]),
     "pnode_circulant_inverse": (C.c_int, [_vp, _i, _d, _vp, _i, _vp, _vp]),
     "pnode_peak_fma": (C.c_int, [_i, _i, C.POINTER(_d), C.POINTER(C.c_float)]),

@@ -16,7 +16,7 @@ UNITS = [("vecops.cu", "vecops.o", []), ("mlp_rk.cu", "mlp_rk.o", ["-DPNODE_MLP_
          ("mlp_rk.cu", "mlp_rk_p1.o", ["-DPNODE_MLP_PART=1"]), ("mlp_rk.cu", "mlp_rk_p2.o", ["-DPNODE_MLP_PART=2"]),
          ("mlp_rk.cu", "mlp_rk_p3.o", ["-DPNODE_MLP_PART=3"]), ("cnf_rk.cu", "cnf_rk.o", []),
          ("bn_relu.cu", "bn_relu.o", []), ("umma_gemm.cu", "umma_gemm.o", []),
-         ("dense_mlp.cu", "dense_mlp.o", []), ("conv_mma.cu", "conv_mma.o", []), ("conv_block.cu", "conv_block_f32.o", ["-DPNODE_CB_PART=1"]),
+         ("dense_mlp.cu", "dense_mlp.o", []), ("cnf_net.cu", "cnf_net.o", []), ("conv_mma.cu", "conv_mma.o", []), ("conv_block.cu", "conv_block_f32.o", ["-DPNODE_CB_PART=1"]),
          ("conv_block.cu", "conv_block_f64.o", ["-DPNODE_CB_PART=2"])]
 SOURCES = sorted({u[0] for u in UNITS})
 HEADERS = ["common.cuh", "umma.cuh", "pdl.cuh", "f32x2.cuh", "graph_cache.cuh", os.path.join("..", "..", "include", "pnode_b200.h")]

@@ -243,19 +243,28 @@ class FusedMlpRK:
 
 
 class CnfSpec:
-    def __init__(self, odefunc, layer1, layer2, batch, dim, hidden):
-        self.odefunc, self.l1, self.l2 = odefunc, layer1, layer2
-        self.batch, self.dim, self.hidden = batch, dim, hidden
+    """A recognised FFJORD right-hand side: ODEfunc `odefunc` over L ConcatSquashLinear `layers` (widths `dims`, dims[0] =
+    dims[L] = D) and a batch of B samples.  `l1`, `l2`, `hidden` describe the two-layer shape of the fused sweeps."""
+
+    def __init__(self, odefunc, layers, batch, dim):
+        self.odefunc, self.layers = odefunc, list(layers)
+        self.batch, self.dim = batch, dim
+        self.dims = [dim] + [m._layer.out_features for m in self.layers]
+        self.l1, self.l2, self.hidden = self.layers[0], self.layers[-1], self.dims[1]
         self.t_via_f32 = 1
+
+    @staticmethod
+    def layer_params(m):
+        return [m._layer.weight, m._layer.bias, m._hyper_bias.weight, m._hyper_gate.weight, m._hyper_gate.bias]
 
     def params(self):
         out = []
-        for l in (self.l1, self.l2):
-            out += [l._layer.weight, l._layer.bias, l._hyper_bias.weight, l._hyper_gate.weight, l._hyper_gate.bias]
+        for m in self.layers:
+            out += self.layer_params(m)
         return out
 
 
-_CNF_RECOGNISED = {}  # (id(diffeq), dim, hidden, dtype, device) -> True once the numerical probe has passed
+_CNF_RECOGNISED = {}  # (id(odefunc), id(diffeq), dims, dtype, device) -> t_via_f32 once the numerical probe has passed
 
 
 def _is_concatsquash(m):
@@ -265,10 +274,39 @@ def _is_concatsquash(m):
             and m._hyper_gate.in_features == 1)
 
 
+def cnf_closed_form(layers, z, e, t):
+    """(f, div) of the ConcatSquash network at time tensor t, the Hutchinson trace div = e^T (df/dz) e formed as the forward
+    tangent of e -- the formula csrc/cnf_net.cu evaluates (and, for two layers, csrc/cnf_rk.cu)."""
+    x, v = z, e
+    for l, m in enumerate(layers):
+        gam = torch.sigmoid(m._hyper_gate(t.view(1, 1)))
+        a = m._layer(x) * gam + m._hyper_bias(t.view(1, 1))
+        u = (v @ m._layer.weight.T) * gam
+        if l < len(layers) - 1:
+            x = torch.nn.functional.softplus(a)
+            v = torch.where(a > 20, torch.ones_like(a), torch.sigmoid(a)) * u
+    return a, (e * u).sum(1)
+
+
+def hutchinson_probe(bf, batch, dim, dtype, device):
+    """The Hutchinson probe of ODEfunc `bf` as the kernels read it.  When absent it is drawn the way the module draws it in
+    the first evaluation of a solve (odefunc.py:359-364); it is kept on the module in the state's dtype and device."""
+    if getattr(bf, "_e", None) is None:
+        z0 = torch.empty(batch, dim, dtype=dtype, device=device)
+        bf._e = torch.randint(0, 2, z0.shape, device=device).to(z0) * 2 - 1 if getattr(bf, "rademacher", False) \
+            else torch.randn_like(z0)
+    e = bf._e
+    if e.dtype != dtype or e.device != device or not e.is_contiguous():
+        e = e.to(device=device, dtype=dtype).contiguous()
+        bf._e = e
+    return e
+
+
 def recognise_cnf(func, u_meta):
-    """Match the object graph cnf.py:72-80 builds -- FlattenFunc(base_func=ODEfunc(diffeq=ODEnet(two ConcatSquashLinear +
-    Softplus), divergence_approx, residual=False), y0=(z [B,D], logp [B,1])) -- by duck typing, then confirm with a numerical
-    probe that func(t, y) equals the closed form the kernel evaluates (once per diffeq module)."""
+    """Match the object graph cnf.py:72-80 builds -- FlattenFunc(base_func=ODEfunc(diffeq=ODEnet(L >= 1 ConcatSquashLinear
+    layers with Softplus between them), divergence_approx, residual=False), y0=(z [B,D], logp [B,1])) -- by duck typing,
+    then confirm with a numerical probe that func(t, y) equals cnf_closed_form (once per diffeq module).  Which runner
+    evaluates it (the two-layer fused sweeps or the evaluator of any depth) is decided where the runner is chosen."""
     bf, y0 = getattr(func, "base_func", None), getattr(func, "y0", None)
     if bf is None or not isinstance(y0, (tuple, list)) or len(y0) != 2 or not u_meta.is_cuda:
         return None
@@ -278,31 +316,34 @@ def recognise_cnf(func, u_meta):
     net = getattr(bf, "diffeq", None)
     layers = getattr(net, "layers", None)
     acts = getattr(net, "activation_fns", None)
-    if layers is None or acts is None or len(layers) != 2 or len(acts) != 1 or getattr(net, "num_squeeze", 0) != 0:
+    if layers is None or acts is None or len(layers) < 1 or len(acts) != len(layers) - 1 or \
+            getattr(net, "num_squeeze", 0) != 0:
         return None
-    if not all(_is_concatsquash(l) for l in layers) or not isinstance(acts[0], nn.Softplus):
+    if not all(_is_concatsquash(l) for l in layers) or not all(isinstance(a, nn.Softplus) for a in acts):
         return None
-    if acts[0].beta != 1 or acts[0].threshold != 20 or getattr(bf, "residual", False):
+    if any(a.beta != 1 or a.threshold != 20 for a in acts) or getattr(bf, "residual", False):
         return None
     if getattr(getattr(bf, "divergence_fn", None), "__name__", "") != "divergence_approx":
         return None
     B, D = z0.shape
-    l1, l2 = layers
-    H = l1._layer.out_features
-    if l1._layer.in_features != D or l2._layer.in_features != H or l2._layer.out_features != D:
+    layers = list(layers)
+    if layers[0]._layer.in_features != D or layers[-1]._layer.out_features != D or \
+            any(a._layer.out_features != b._layer.in_features for a, b in zip(layers[:-1], layers[1:])):
         return None
-    spec = CnfSpec(bf, l1, l2, B, D, H)
+    spec = CnfSpec(bf, layers, B, D)
     plist = [p for p in func.parameters() if p.requires_grad]
     want = spec.params()
     if len(plist) != len(want) or any(a is not b for a, b in zip(plist, want)):
         return None
     if any(p.dtype != u_meta.dtype or p.device != u_meta.device or not p.is_contiguous() for p in want):
         return None
-    key = (id(bf), id(net), D, H, u_meta.dtype, str(u_meta.device))
+    key = (id(bf), id(net), tuple(spec.dims), u_meta.dtype, str(u_meta.device))
     if key not in _CNF_RECOGNISED:
         # probe through the user's module itself (FlattenFunc -> ODEfunc -> ODEnet), on a small batch, at times that are
         # not representable in float32 so that the module's handling of `t` is observable
         e_saved = getattr(bf, "_e", None)
+        nevals = getattr(bf, "_num_evals", None)
+        nevals = nevals.clone() if isinstance(nevals, torch.Tensor) else None
         nb = min(B, 8)
         try:
             with torch.no_grad():
@@ -318,14 +359,8 @@ def recognise_cnf(func, u_meta):
                         got = type(func)(bf, (z, torch.zeros(nb, 1).to(u_meta)))(tval, torch.cat((z.reshape(-1),
                                                                                   torch.zeros(nb).to(u_meta))))
                         t = torch.tensor(tval).to(u_meta) if via_f32 else torch.tensor(tval, dtype=torch.float64).to(u_meta)
-                        g1 = torch.sigmoid(l1._hyper_gate(t.view(1, 1)))
-                        g2 = torch.sigmoid(l2._hyper_gate(t.view(1, 1)))
-                        a = l1._layer(z) * g1 + l1._hyper_bias(t.view(1, 1))
-                        sp_, sg = torch.nn.functional.softplus(a), torch.sigmoid(a)
-                        dz2 = l2._layer(sp_) * g2 + l2._hyper_bias(t.view(1, 1))
-                        w = (g2 * e) @ l2._layer.weight
-                        q = e @ l1._layer.weight.T
-                        ref = torch.cat((dz2.reshape(-1), -(g1 * sg * w * q).sum(1)))
+                        f, div = cnf_closed_form(layers, z, e, t)
+                        ref = torch.cat((f.reshape(-1), -div))
                         ok = ok and got.shape == ref.shape and torch.allclose(got.detach(), ref, rtol=tol, atol=tol)
                     if ok:
                         verdict = via_f32
@@ -334,6 +369,8 @@ def recognise_cnf(func, u_meta):
             verdict = None
         finally:
             bf._e = e_saved
+            if nevals is not None:
+                bf._num_evals.copy_(nevals)  # the probe is not an evaluation of the user's solve
         if verdict is None:
             return None
         _CNF_RECOGNISED[key] = verdict
@@ -363,20 +400,12 @@ class FusedCnfRK:
 
     @staticmethod
     def supported(spec, scheme, dtype):
-        return bool(_lib.load().pnode_cnf_rk_supported(spec.dim, spec.hidden, dtype_code(dtype), scheme.s))
+        return len(spec.layers) == 2 and bool(_lib.load().pnode_cnf_rk_supported(spec.dim, spec.hidden, dtype_code(dtype),
+                                                                                  scheme.s))
 
     def _desc(self):
         sp = self.spec
-        bf = sp.odefunc
-        if getattr(bf, "_e", None) is None:
-            # the reference samples the Hutchinson probe inside the first RHS evaluation of a solve (odefunc.py:359-364)
-            z0 = torch.empty(sp.batch, sp.dim, dtype=self.dtype, device=self.device)
-            bf._e = torch.randint(0, 2, z0.shape, device=self.device).to(z0) * 2 - 1 if getattr(bf, "rademacher", False) \
-                else torch.randn_like(z0)
-        e = bf._e
-        if e.dtype != self.dtype or e.device != self.device or not e.is_contiguous():
-            e = e.to(device=self.device, dtype=self.dtype).contiguous()
-            bf._e = e
+        e = hutchinson_probe(sp.odefunc, sp.batch, sp.dim, self.dtype, self.device)
         d = _lib.CnfDesc()
         d.dim, d.hidden, d.dtype, d.t_via_f32 = sp.dim, sp.hidden, self.code, sp.t_via_f32
         names = ("d_w1", "d_b1", "d_hb1", "d_hgw1", "d_hgb1", "d_w2", "d_b2", "d_hb2", "d_hgw2", "d_hgb2")

@@ -18,6 +18,7 @@ import torch
 import torch.nn as nn
 
 from . import tableaux
+from .cnfnet import CnfNetCallbacks
 from .controller import TimeLoop
 from .device import DeviceOps
 from .convblock import ConvBlockCallbacks, recognise_convblock
@@ -103,7 +104,7 @@ class ODEPetsc(object):
         self._fused_checked_for = None
         self._cb_ex = self._cb_im = self._imp = None
         self._loop = None
-        self.path = None  # "fused-mlp-rk" | "generic": which engine ran the last odeint
+        self.path = None  # "fused-mlp-rk" | "fused-cnf-rk" | "generic[+<evaluator>-rhs]": which engine ran the last odeint
 
     # ------------------------------------------------------------------------------------------------------------
     def setupTS(self, u_tensor, func, step_size=0.01, enable_adjoint=True, implicit_form=False, use_dlpack=True,
@@ -162,6 +163,13 @@ class ODEPetsc(object):
                         self._cb_im = cb
                     self._cb_ex = cb
                     self._rhs_kind = "dense-mlp"
+                if spec is None and not imex_form:
+                    # FFJORD network of any depth: tensor-core evaluator with the trace and its adjoint in closed form (the
+                    # two-layer shapes of the fused sweeps still take those where _fused_runner picks them)
+                    cnf = recognise_cnf(self.funcEX, u_tensor)
+                    if cnf is not None and CnfNetCallbacks.supported(cnf, u_tensor.dtype):
+                        self._cb_ex = self._cb_im = CnfNetCallbacks(self.funcEX, self.tensor_size, cnf)
+                        self._rhs_kind = "cnf-net"
                 if imex_form:
                     col = recognise_circulant(self.funcIM, u_tensor)
                     if col is not None:
