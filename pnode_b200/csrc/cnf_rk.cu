@@ -69,7 +69,8 @@ __device__ __forceinline__ void softplus_sigmoid(float a, float &s, float &sg) {
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(d));
     asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l) : "f"(d));
     sg = a >= 0.0f ? r : E * r;
-    // no threshold branch: for a > 20, E < 2^-28 so d rounds to 1, lg2(1) = +0 and s = a exactly, as torch's Softplus returns
+    // no threshold branch: for a > 20, E < 2^-28 so d rounds to 1, lg2(1) = +0 and s = a exactly, and rcp(1) = 1 so sg = 1
+    // exactly -- the value, slope and zero curvature of torch's Softplus above its threshold
     s = fmaf(l, 0.6931471805599453f, fmaxf(a, 0.0f));
 }
 // two trajectories at once: the MUFU part is per half, the arithmetic around it packed
@@ -88,10 +89,12 @@ __device__ __forceinline__ void softplus_sigmoid(F2 a, F2 &s, F2 &sg) {
     s = fma(pk(l0, l1), 0.6931471805599453f, pk(fmaxf(a0, 0.0f), fmaxf(a1, 0.0f)));
 }
 __device__ __forceinline__ void softplus_sigmoid(double a, double &s, double &sg) {
-    const double E = exp(-fabs(a));
+    // torch's threshold: above 20, E = 0 makes s = a and sg = 1 exactly -- the value, slope and zero curvature of the
+    // identity (sigmoid(20) = 1 - 2e-9 would miss the fp64 parity bar), so the adjoint's 1 - sg is exactly 0
+    const double E = a > 20.0 ? 0.0 : exp(-fabs(a));
     const double r = 1.0 / (1.0 + E);
     sg = a >= 0.0 ? r : E * r;
-    s = a > 20.0 ? a : fmax(a, 0.0) + log1p(E);
+    s = fmax(a, 0.0) + log1p(E);
 }
 
 // shared-memory image of the model for one launch

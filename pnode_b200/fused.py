@@ -6,6 +6,7 @@ Currently fused: tiny-state MLPs  f(t,y) = Linear(H,d)(tanh(Linear(d,H)(phi(y)))
 examples-pnode/ode_demo_petsc.py:207-230 -- under any fixed-step explicit RK scheme (csrc/mlp_rk.cu).
 """
 import ctypes as C
+import weakref
 
 import numpy as np
 import torch
@@ -264,7 +265,9 @@ class CnfSpec:
         return out
 
 
-_CNF_RECOGNISED = {}  # (id(odefunc), id(diffeq), dims, dtype, device) -> t_via_f32 once the numerical probe has passed
+# odefunc -> {(id(diffeq), dims, dtype, device): (weakref to diffeq, t_via_f32)} once the numerical probe has passed.  Weak in
+# both modules: a verdict must not pass to a new module that CPython places at the address of a freed one.
+_CNF_RECOGNISED = weakref.WeakKeyDictionary()
 
 
 def _is_concatsquash(m):
@@ -337,8 +340,9 @@ def recognise_cnf(func, u_meta):
         return None
     if any(p.dtype != u_meta.dtype or p.device != u_meta.device or not p.is_contiguous() for p in want):
         return None
-    key = (id(bf), id(net), tuple(spec.dims), u_meta.dtype, str(u_meta.device))
-    if key not in _CNF_RECOGNISED:
+    seen = _CNF_RECOGNISED.setdefault(bf, {})
+    key = (id(net), tuple(spec.dims), u_meta.dtype, str(u_meta.device))
+    if key not in seen or seen[key][0]() is not net:
         # probe through the user's module itself (FlattenFunc -> ODEfunc -> ODEnet), on a small batch, at times that are
         # not representable in float32 so that the module's handling of `t` is observable
         e_saved = getattr(bf, "_e", None)
@@ -373,8 +377,8 @@ def recognise_cnf(func, u_meta):
                 bf._num_evals.copy_(nevals)  # the probe is not an evaluation of the user's solve
         if verdict is None:
             return None
-        _CNF_RECOGNISED[key] = verdict
-    spec.t_via_f32 = _CNF_RECOGNISED[key]
+        seen[key] = (weakref.ref(net), verdict)
+    spec.t_via_f32 = seen[key][1]
     return spec
 
 

@@ -21,8 +21,9 @@ def _softplus_sigmoid(a):
     return sp, s
 
 
-def forward(layers, z, e, tau):
-    """F = (f, -div) flattened like FlattenFunc, and what the adjoint needs per layer."""
+def forward(layers, z, e, tau, abs_terms=False):
+    """F = (f, -div) flattened like FlattenFunc, and what the adjoint needs per layer.  With abs_terms, also the sum of the
+    absolute values of the terms of the last layer's sums (the scale of each entry's rounding error)."""
     gs = gates(layers, tau)
     x, v = z, e
     cache = []
@@ -37,15 +38,28 @@ def forward(layers, z, e, tau):
         if l < len(layers) - 1:
             x, v = sp, s * u
     div = (e * u).sum(1)
-    return torch.cat((a.reshape(-1), -div)), cache
+    F = torch.cat((a.reshape(-1), -div))
+    if not abs_terms:
+        return F, cache
+    aW = W.abs()
+    f_abs = gam.abs() * (x.abs() @ aW.T + b.abs()) + c.abs()
+    div_abs = (e.abs() * gam.abs() * (v.abs() @ aW.T)).sum(1)
+    return F, cache, torch.cat((f_abs.reshape(-1), div_abs))
 
 
-def vjp(layers, cache, e, w, tau):
-    """(J^T w flattened, [[dW, db, dhbw, dhgw, dhgb] per layer]) for the cotangent w = (w_z, w_logp)."""
+def vjp(layers, cache, e, w, tau, abs_terms=False):
+    """(J^T w flattened, [[dW, db, dhbw, dhgw, dhgb] per layer]) for the cotangent w = (w_z, w_logp).
+
+    With abs_terms, also the same two results with the operands of every product and every sum in absolute value -- for
+    example |Pbar|^T |x| + |Qbar|^T |v| for dW and sum |Pbar| for db -- the scale against which each entry's rounding error
+    is measured."""
     B, D = e.shape
     wz, wl = w[:B * D].view(B, D), w[B * D:]
     abar, ubar = wz, -wl[:, None] * e
     grads = [None] * len(layers)
+    if abs_terms:
+        abar_a, ubar_a = abar.abs(), ubar.abs()
+        grads_a = [None] * len(layers)
     for l in range(len(layers) - 1, -1, -1):
         k, m = cache[l], layers[l]
         gam = k["gam"]
@@ -56,8 +70,22 @@ def vjp(layers, cache, e, w, tau):
         cbar = abar.sum(0)
         gg = gbar * gam * (1 - gam)
         grads[l] = [dW, db, (cbar * tau)[:, None], (gg * tau)[:, None], gg]
-        xb, vb = Pb @ m._layer.weight, Qb @ m._layer.weight
+        W = m._layer.weight
+        xb, vb = Pb @ W, Qb @ W
+        if abs_terms:
+            g_a, aW = gam.abs(), W.abs()
+            Pa, Qa = g_a * abar_a, g_a * ubar_a
+            gg_a = (abar_a * k["P"].abs() + ubar_a * k["Q"].abs()).sum(0) * g_a * (1 - gam).abs()
+            grads_a[l] = [Pa.T @ k["x"].abs() + Qa.T @ k["v"].abs(), Pa.sum(0), (abar_a.sum(0) * abs(tau))[:, None],
+                          (gg_a * abs(tau))[:, None], gg_a]
+            xb_a, vb_a = Pa @ aW, Qa @ aW
         if l > 0:
             s, u = cache[l - 1]["s"], cache[l - 1]["u"]
             abar, ubar = s * xb + s * (1 - s) * u * vb, s * vb
-    return torch.cat((xb.reshape(-1), torch.zeros(B, dtype=w.dtype, device=w.device))), grads
+            if abs_terms:
+                abar_a, ubar_a = s * xb_a + s * (1 - s) * u.abs() * vb_a, s * vb_a
+    zeros = torch.zeros(B, dtype=w.dtype, device=w.device)
+    jtw = torch.cat((xb.reshape(-1), zeros))
+    if not abs_terms:
+        return jtw, grads
+    return jtw, grads, torch.cat((xb_a.reshape(-1), zeros)), grads_a

@@ -79,6 +79,22 @@ class ODEfunc(nn.Module):
         return (dy, -divergence)
 
 
+class ODEfuncT64(ODEfunc):
+    """ODEfunc that keeps t in double precision (the reference's module rounds it through float32)."""
+
+    def forward(self, t, states):
+        y = states[0]
+        self._num_evals += 1
+        t = torch.tensor(t, dtype=torch.float64).type_as(y)
+        if self._e is None:
+            self._e = torch.randn_like(y)
+        with torch.set_grad_enabled(True):
+            y.requires_grad_(True)
+            dy = self.diffeq(t, y)
+            divergence = self.divergence_fn(dy, y, e=self._e).view(y.shape[0], 1)
+        return (dy, -divergence)
+
+
 class FlattenFunc(nn.Module):
     """lib/layers/cnf.py:123-150: the state handed to ODEPetsc is cat(z.view(-1), logp.view(-1))."""
 
@@ -96,10 +112,11 @@ class FlattenFunc(nn.Module):
         return torch.cat([o.contiguous().view(-1) for o in out])
 
 
-def CNFFunc(batch, dim=6, hidden_dims=(60,), dtype=torch.float32, seed=0, device="cpu"):
-    """FlattenFunc(ODEfunc(ODEnet)) with the Hutchinson probe already fixed (seeded) -- what cnf.py:72-80 builds."""
+def CNFFunc(batch, dim=6, hidden_dims=(60,), dtype=torch.float32, seed=0, device="cpu", t_via_f32=True):
+    """FlattenFunc(ODEfunc(ODEnet)) with the Hutchinson probe already fixed (seeded) -- what cnf.py:72-80 builds.  With
+    t_via_f32=False the ODEfunc keeps t in double precision (ODEfuncT64) instead of rounding it through float32."""
     torch.manual_seed(seed)
-    odefunc = ODEfunc(ODEnet(hidden_dims, dim).to(dtype))
+    odefunc = (ODEfunc if t_via_f32 else ODEfuncT64)(ODEnet(hidden_dims, dim).to(dtype))
     g = torch.Generator().manual_seed(seed + 1)
     odefunc._e = torch.randn(batch, dim, generator=g, dtype=torch.float64).to(dtype)
     y0 = (torch.zeros(batch, dim, dtype=dtype), torch.zeros(batch, 1, dtype=dtype))

@@ -6,27 +6,11 @@ import pytest
 import torch
 
 import _cnf_net_model as model
-from _workloads import CNFFunc, ODEfunc
-
-
-class ODEfuncT64(ODEfunc):
-    """ODEfunc that keeps t in double precision (the reference's module rounds it through float32)."""
-
-    def forward(self, t, states):
-        y = states[0]
-        self._num_evals += 1
-        t = torch.tensor(t, dtype=torch.float64).type_as(y)
-        with torch.set_grad_enabled(True):
-            y.requires_grad_(True)
-            dy = self.diffeq(t, y)
-            divergence = self.divergence_fn(dy, y, e=self._e).view(y.shape[0], 1)
-        return (dy, -divergence)
+from _workloads import CNFFunc
 
 
 def _case(B, D, hidden, seed, via_f32=True, saturate=0):
-    func = CNFFunc(B, D, hidden, dtype=torch.float64, seed=seed)
-    if not via_f32:
-        func.base_func.__class__ = ODEfuncT64
+    func = CNFFunc(B, D, hidden, dtype=torch.float64, seed=seed, t_via_f32=via_f32)
     layers = list(func.base_func.diffeq.layers)
     if saturate:
         with torch.no_grad():  # push the first units of the first layer just past the softplus threshold (a ~ 21)

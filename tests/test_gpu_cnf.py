@@ -80,15 +80,20 @@ def test_rejections_and_multiple_output_times_fp64():
     _compare(p, o, 2e-9)  # weights x4: the flow amplifies rounding differences ~20x more than the default model
 
 
-@pytest.mark.parametrize("method,argv", [("rk4", ["-ts_adapt_type", "none"]), ("dopri5", ["-ts_adapt_type", "none"]),
-                                         ("bosh3", []), ("euler", [])])
-def test_other_schemes_fused_fp64(method, argv):
+@pytest.mark.parametrize("method,argv,t_via_f32", [
+    pytest.param("rk4", ["-ts_adapt_type", "none"], True, id="rk4-argv0"),
+    pytest.param("dopri5", ["-ts_adapt_type", "none"], True, id="dopri5-argv1"),
+    pytest.param("bosh3", [], True, id="bosh3-argv2"),
+    pytest.param("euler", [], True, id="euler-argv3"),
+    # a module that keeps t in fp64: every stage time but the first is off the fp32 grid
+    pytest.param("dopri5", ["-ts_adapt_type", "none"], False, id="dopri5-t-f64")])
+def test_other_schemes_fused_fp64(method, argv, t_via_f32):
     B = 64
-    func = CNFFunc(B, 6, (60,), dtype=torch.float64, seed=5)
+    func = CNFFunc(B, 6, (60,), dtype=torch.float64, seed=5, t_via_f32=t_via_f32)
     u0, gout = _inputs(B, 6, 3, torch.float64)
-    t = torch.tensor([0.0, 0.5, 1.0], dtype=torch.float64)
+    t = torch.tensor([0.0, 0.5, 1.0], dtype=torch.float64) + (0.0 if t_via_f32 else 0.3)
     o, p = _pair(argv, func, u0, t, gout, method, 0.25)
-    assert p[3].path == "fused-cnf-rk"
+    assert p[3].path == "fused-cnf-rk" and p[3]._fused.spec.t_via_f32 == int(t_via_f32)
     _compare(p, o, 1e-10)
 
 

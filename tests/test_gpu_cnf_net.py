@@ -103,17 +103,19 @@ def test_dopri5_adaptive_takes_the_oracle_s_steps(dtype, ts_tol):
     _compare(p, o, TOL[dtype])
 
 
-@pytest.mark.parametrize("method,argv,tol", [("bosh3", [], 1e-10), ("imex", FIXED, 1e-10),
-                                             ("cn", FIXED + ["-ksp_rtol", "1e-13", "-snes_rtol", "1e-13"], 1e-8)],
-                         ids=["3bs-adaptive", "arkimex", "cn"])
-def test_other_schemes_fp64(method, argv, tol):
+@pytest.mark.parametrize("method,argv,tol,t_via_f32", [
+    ("bosh3", [], 1e-10, True), ("imex", FIXED, 1e-10, True),
+    ("cn", FIXED + ["-ksp_rtol", "1e-13", "-snes_rtol", "1e-13"], 1e-8, True), ("bosh3", [], 1e-10, False)],
+                         ids=["3bs-adaptive", "arkimex", "cn", "3bs-adaptive-t-f64"])
+def test_other_schemes_fp64(method, argv, tol, t_via_f32):
+    """t_via_f32=False: a module that keeps t in fp64, from a start time off the fp32 grid."""
     B, D = 40, 5
-    func = CNFFunc(B, D, (37, 129), dtype=torch.float64, seed=4)
+    func = CNFFunc(B, D, (37, 129), dtype=torch.float64, seed=4, t_via_f32=t_via_f32)
     u0, gout = _inputs(B, D, 3, torch.float64)
-    t = torch.tensor([0.0, 0.5, 1.0], dtype=torch.float64)
+    t = torch.tensor([0.0, 0.5, 1.0], dtype=torch.float64) + (0.0 if t_via_f32 else 0.3)
     o = _oracle(argv, func, u0, t, gout, method, 0.25)
     p = _mine(argv, func, u0, t, gout, method, 0.25)
-    assert p[3].path == PATH
+    assert p[3].path == PATH and p[3]._cb_ex.spec.t_via_f32 == int(t_via_f32)
     _compare(p, o, tol)
 
 
