@@ -384,14 +384,6 @@ int pnode_convblock_vjp(const pnode_convblock_desc *desc, const void *d_x, const
  * pnode_convblock_forward / _vjp; additionally d_wbuf (pnode_convmma_weight_bytes) holds the weight operands written by
  * pnode_convmma_prepare once per solve, and d_work is needed by the forward as well.  N*H*W <= 65536, channel counts
  * multiples of 4 and >= 8, kernels 1x1 / (1,3) / (3,1) with "same" padding. */
-/* Optional (off by default): the forward / vjp entry points of both conv evaluators can replay their launch sequence from a
- * CUDA graph once they have seen the same arguments twice (csrc/graph_cache.cuh; single-GPU descriptors only; a call made
- * while the caller's stream is being captured launches directly).  On with pnode_graph_cache_enable(1), PNODE_CONV_GRAPHS=1
- * or the option -pnode_conv_graphs 1.  Counters since load: sequences replayed, graphs recorded, sequences launched
- * directly.  pnode_graph_cache_stats returns 1 while the cache is on, 0 when off, -1 before the first call. */
-int pnode_graph_cache_enable(int on);
-int pnode_graph_cache_stats(int64_t *replays, int64_t *recorded, int64_t *direct);
-
 int64_t pnode_convmma_act_bytes(const pnode_convblock_desc *desc);     /* -1: unsupported shape (pnode_last_error) */
 int64_t pnode_convmma_work_bytes(const pnode_convblock_desc *desc);
 int64_t pnode_convmma_weight_bytes(const pnode_convblock_desc *desc);

@@ -105,8 +105,6 @@ _SIGNATURES = {
     "pnode_mlp_rk_forward_so": (C.c_int, [C.POINTER(MlpDesc), C.POINTER(RKTableau), _vp, _i64, _vp, _i, _vp, _vp, _vp]),
     "pnode_mlp_rk_adjoint_so": (C.c_int, [C.POINTER(MlpDesc), C.POINTER(RKTableau), _i64, _vp, _i, _i, _vp, _vp, _vp, _vp,
                                           _vp, _vp, _i, _i, C.c_uint64, _vp]),
-    "pnode_graph_cache_stats": (C.c_int, [_vp, _vp, _vp]),
-    "pnode_graph_cache_enable": (C.c_int, [_i]),
     "pnode_cnf_rk_supported": (C.c_int, [_i, _i, _i, _i]),
     "pnode_cnf_rk_attempt": (C.c_int, [C.POINTER(CnfDesc), C.POINTER(RKTableau), _vp, _vp, _i64, _d, _d, _vp, _vp, _vp, _d,
                                        _d, _vp, _vp, _vp]),

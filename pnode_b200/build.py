@@ -19,7 +19,7 @@ UNITS = [("vecops.cu", "vecops.o", []), ("mlp_rk.cu", "mlp_rk.o", ["-DPNODE_MLP_
          ("dense_mlp.cu", "dense_mlp.o", []), ("cnf_net.cu", "cnf_net.o", []), ("conv_mma.cu", "conv_mma.o", []), ("conv_block.cu", "conv_block_f32.o", ["-DPNODE_CB_PART=1"]),
          ("conv_block.cu", "conv_block_f64.o", ["-DPNODE_CB_PART=2"])]
 SOURCES = sorted({u[0] for u in UNITS})
-HEADERS = ["common.cuh", "umma.cuh", "pdl.cuh", "f32x2.cuh", "graph_cache.cuh", os.path.join("..", "..", "include", "pnode_b200.h")]
+HEADERS = ["common.cuh", "umma.cuh", "pdl.cuh", "f32x2.cuh", os.path.join("..", "..", "include", "pnode_b200.h")]
 LIB = os.path.join(CSRC, "libpnode_b200.so")
 NVCC_FLAGS = ["-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-Xcompiler", "-fPIC"]
 

@@ -98,66 +98,61 @@ class ConvBlockCallbacks(Callbacks):
         dev = self.params[0].device
         self._work = torch.empty(int(self.lib.pnode_bn_work_bytes(cmax)), dtype=torch.uint8, device=dev)
         self.launches = 0
-        # native whole-chain kernels (csrc/conv_block.cu) when the shapes are the SqueezeNext ones
-        self.native = False
+        self.native = self.mma = False
         self._desc = None
         self._cwork = None
+        picked = self._pick_evaluator(tensor_size)
+        if picked is None:
+            return
         from .options import Options
 
-        if Options().hasName("pnode_conv_graphs"):  # optional per-call CUDA graphs of the launch sequences (csrc/graph_cache.cuh)
-            on = Options().getString("pnode_conv_graphs", "0") not in ("0", "false", "no")
-            _lib.check(self.lib.pnode_graph_cache_enable(int(on)))
+        self.mma, self._desc, self._act_bytes, work_bytes = picked
+        self.native = True
+        self._cwork = torch.empty(work_bytes, dtype=torch.uint8, device=dev)
+        self._act0 = torch.empty(self._act_bytes, dtype=torch.uint8, device=dev)  # for evaluations that are not kept
+        # Forward evaluations keep their activation set (z_1..z_L + batch statistics: the forward's by-product) so that the
+        # adjoint stage at the same point skips the module's forward re-evaluation; bounded by a byte budget.
+        self._saved = {}
+        self._saved_bytes = 0
+        self._save_budget = int(float(Options().getString("pnode_convblock_save_mb", "8192")) * (1 << 20))
+        self.reused_activations = 0
+        self._keep = True
+        self._comm = None
+        if self.mma:
+            self._wbuf = torch.empty(int(self.lib.pnode_convmma_weight_bytes(C.byref(self._desc))), dtype=torch.uint8,
+                                     device=dev)
+            self._wbuf_for = None
+
+    def _pick_evaluator(self, tensor_size):
+        """(mma, descriptor, activation bytes, work bytes) of the native evaluator that takes this shape, or None: library
+        convolutions."""
+        from .options import Options
+
+        off = ("0", "false", "no")
         mode = Options().getString("pnode_convblock_native", "auto")  # auto | 1 (whenever the shape is supported) | 0
+        if len(self.layers) > _lib.CONV_MAX_LAYERS or len(tensor_size) != 4 or mode in off:
+            return None
         # Tensor-core evaluator (csrc/conv_mma.cu, fp32 as 3xTF32) for GEMM-sized shapes: every layer at least 32 channels
         # wide (the CIFAR blocks [256,128,8,8] and [256,256,4,4]).  -pnode_convblock_mma auto | 1 (whenever supported) | 0
-        self.mma = False
         mma_mode = Options().getString("pnode_convblock_mma", "auto")
-        if (len(self.layers) <= _lib.CONV_MAX_LAYERS and len(tensor_size) == 4 and self.params[0].dtype == torch.float32
-                and mma_mode not in ("0", "false", "no") and mode not in ("0", "false", "no")):
+        if self.params[0].dtype == torch.float32 and mma_mode not in off:
             wide = min(min(c.in_channels, c.out_channels) for c, _ in self.layers) >= 32
             if wide or mma_mode in ("1", "true", "yes", "force"):
                 desc = self._make_desc()
                 nact = int(self.lib.pnode_convmma_act_bytes(C.byref(desc)))
                 if nact >= 0 and int(self.lib.pnode_convmma_param_count(C.byref(desc))) == self.nparams:
-                    self.mma = True
-                    self.native = True
-                    self._desc = desc
-                    self._act_bytes = nact
-                    self._cwork = torch.empty(int(self.lib.pnode_convmma_work_bytes(C.byref(desc))), dtype=torch.uint8,
-                                              device=dev)
-                    self._wbuf = torch.empty(int(self.lib.pnode_convmma_weight_bytes(C.byref(desc))), dtype=torch.uint8,
-                                             device=dev)
-                    self._wbuf_for = None
-                    self._act0 = torch.empty(nact, dtype=torch.uint8, device=dev)
-                    self._saved = {}
-                    self._saved_bytes = 0
-                    self._save_budget = int(float(Options().getString("pnode_convblock_save_mb", "8192")) * (1 << 20))
-                    self.reused_activations = 0
-                    self._keep = True
-                    self._comm = None
-        if (not self.mma and len(self.layers) <= _lib.CONV_MAX_LAYERS and len(tensor_size) == 4
-                and mode not in ("0", "false", "no")):
-            desc = self._make_desc()
-            nact = int(self.lib.pnode_convblock_act_bytes(C.byref(desc)))
-            # The native kernels give one thread 4 pixels x 16 output channels: they need pixels to fill the machine.  The
-            # last CIFAR block ([256,256,4,4]: 4096 pixels, 256 channels) is a small GEMM per layer -- measured 2.3x slower
-            # than the library GEMM convolutions there (tools/time_convblock.py), 1.7x-4.2x faster on the other three.
-            pixels = int(tensor_size[0]) * int(tensor_size[2]) * int(tensor_size[3])
-            enough = pixels >= self.NATIVE_MIN_PIXELS or mode in ("1", "true", "yes", "force")
-            if nact >= 0 and enough and int(self.lib.pnode_convblock_param_count(C.byref(desc))) == self.nparams:
-                self.native = True
-                self._desc = desc
-                self._act_bytes = nact
-                self._cwork = torch.empty(int(self.lib.pnode_convblock_work_bytes(C.byref(desc))), dtype=torch.uint8, device=dev)
-                self._act0 = torch.empty(nact, dtype=torch.uint8, device=dev)  # activation set of evaluations that are not kept
-                # Forward evaluations keep their activation set (z_1..z_L + batch statistics: the forward's by-product) so
-                # that the adjoint stage at the same point skips the module's forward re-evaluation; bounded by a byte budget.
-                self._saved = {}
-                self._saved_bytes = 0
-                self._save_budget = int(float(Options().getString("pnode_convblock_save_mb", "8192")) * (1 << 20))
-                self.reused_activations = 0
-                self._keep = True
-                self._comm = None
+                    return True, desc, nact, int(self.lib.pnode_convmma_work_bytes(C.byref(desc)))
+        # CUDA-core whole-chain kernels (csrc/conv_block.cu) for the SqueezeNext shapes
+        desc = self._make_desc()
+        nact = int(self.lib.pnode_convblock_act_bytes(C.byref(desc)))
+        # The native kernels give one thread 4 pixels x 16 output channels: they need pixels to fill the machine.  The
+        # last CIFAR block ([256,256,4,4]: 4096 pixels, 256 channels) is a small GEMM per layer -- measured 2.3x slower
+        # than the library GEMM convolutions there (tools/time_convblock.py), 1.7x-4.2x faster on the other three.
+        pixels = int(tensor_size[0]) * int(tensor_size[2]) * int(tensor_size[3])
+        enough = pixels >= self.NATIVE_MIN_PIXELS or mode in ("1", "true", "yes", "force")
+        if nact >= 0 and enough and int(self.lib.pnode_convblock_param_count(C.byref(desc))) == self.nparams:
+            return False, desc, nact, int(self.lib.pnode_convblock_work_bytes(C.byref(desc)))
+        return None
 
     def _make_desc(self):
         d = _lib.ConvBlockDesc()

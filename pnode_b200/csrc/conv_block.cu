@@ -45,7 +45,6 @@
 
 #include "common.cuh"
 #include "f32x2.cuh"
-#include "graph_cache.cuh"
 #include "pdl.cuh"
 
 namespace pnode {
@@ -1625,14 +1624,9 @@ int pnode_convblock_forward(const pnode_convblock_desc *desc, const void *d_x, v
     PNODE_REQUIRE(cb_aligned(d_x) && cb_aligned(d_out) && cb_aligned(d_base) && cb_aligned(d_k) && cb_aligned(d_act),
                   "pnode_convblock_forward: tensors must be 16-byte aligned");
     PNODE_REQUIRE(desc->layer[p.L - 1].cout == desc->layer[0].cin, "pnode_convblock_forward: an ODE right-hand side maps C -> C");
-    auto launch = [&](cudaStream_t st) -> int {
-        if (desc->dtype == PNODE_F32) return run_forward<float>(desc, p, d_x, d_out, d_base, base_coef, k_coef, d_k, d_act, st);
-        return convblock_forward_f64(desc, d_x, d_out, d_base, base_coef, k_coef, d_k, d_act, st);
-    };
-    if (desc->world > 1) return launch(static_cast<cudaStream_t>(stream));  // the collective number changes with every call
-    gcache::Key key;  // csrc/graph_cache.cuh: the launch sequence replays from a CUDA graph once its arguments repeat
-    key.add(3).add(*desc).add(d_x).add(d_out).add(d_base).add(base_coef).add(k_coef).add(d_k).add(d_act);
-    return gcache::run(key, static_cast<cudaStream_t>(stream), launch);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (desc->dtype == PNODE_F32) return run_forward<float>(desc, p, d_x, d_out, d_base, base_coef, k_coef, d_k, d_act, st);
+    return convblock_forward_f64(desc, d_x, d_out, d_base, base_coef, k_coef, d_k, d_act, st);
 }
 
 int pnode_convblock_vjp(const pnode_convblock_desc *desc, const void *d_x, const void *d_w, void *d_vu, void *d_grads,
@@ -1643,15 +1637,10 @@ int pnode_convblock_vjp(const pnode_convblock_desc *desc, const void *d_x, const
     PNODE_REQUIRE(d_x && d_w && d_act && d_work && (d_vu || d_grads), "pnode_convblock_vjp: null argument");
     PNODE_REQUIRE(cb_aligned(d_x) && cb_aligned(d_w) && cb_aligned(d_vu) && cb_aligned(d_act) && cb_aligned(d_work),
                   "pnode_convblock_vjp: tensors must be 16-byte aligned");
-    auto launch = [&](cudaStream_t st) -> int {
-        if (desc->dtype == PNODE_F32)
-            return run_vjp<float>(desc, p, d_x, d_w, d_vu, d_grads, coef, accumulate, d_act, act_valid, d_work, st);
-        return convblock_vjp_f64(desc, d_x, d_w, d_vu, d_grads, coef, accumulate, d_act, act_valid, d_work, st);
-    };
-    if (desc->world > 1) return launch(static_cast<cudaStream_t>(stream));
-    gcache::Key key;
-    key.add(4).add(*desc).add(d_x).add(d_w).add(d_vu).add(d_grads).add(coef).add(accumulate).add(d_act).add(act_valid).add(d_work);
-    return gcache::run(key, static_cast<cudaStream_t>(stream), launch);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (desc->dtype == PNODE_F32)
+        return run_vjp<float>(desc, p, d_x, d_w, d_vu, d_grads, coef, accumulate, d_act, act_valid, d_work, st);
+    return convblock_vjp_f64(desc, d_x, d_w, d_vu, d_grads, coef, accumulate, d_act, act_valid, d_work, st);
 }
 
 }  // extern "C"

@@ -15,7 +15,6 @@
 // forward re-evaluation; batch-sharded runs exchange the statistics of the GLOBAL batch over NVLink peer memory inside the
 // finalize kernels.
 #include "common.cuh"
-#include "graph_cache.cuh"
 #include "umma.cuh"
 
 namespace pnode {
@@ -580,23 +579,6 @@ using cmma::Plan;
 
 extern "C" {
 
-int pnode_graph_cache_stats(int64_t *replays, int64_t *recorded, int64_t *direct) {
-    gcache::Cache &c = gcache::cache();
-    std::lock_guard<std::mutex> lock(c.mu);
-    if (replays) *replays = c.hits;
-    if (recorded) *recorded = c.records;
-    if (direct) *direct = c.direct;
-    return c.enabled;
-}
-
-int pnode_graph_cache_enable(int on) {
-    gcache::Cache &c = gcache::cache();
-    std::lock_guard<std::mutex> lock(c.mu);
-    if (!on) gcache::drop_all(c);
-    c.enabled = on ? 1 : 0;
-    return 0;
-}
-
 int64_t pnode_convmma_act_bytes(const pnode_convblock_desc *desc) {
     Plan p;
     return cmma::make_plan(desc, p) ? -1 : p.act_total;
@@ -637,20 +619,15 @@ int pnode_convmma_forward(const pnode_convblock_desc *desc, const void *d_wbuf, 
     Plan p;
     if (int rc = cmma::make_plan(desc, p)) return rc;
     PNODE_REQUIRE(d_wbuf && d_x && d_act && d_work && (d_out || d_k), "pnode_convmma_forward: null argument");
-    auto launch = [&](cudaStream_t st) -> int {
-        uint8_t *act = (uint8_t *)d_act, *work = (uint8_t *)d_work;
-        if (int rc = cmma::forward_impl(desc, p, (const uint8_t *)d_wbuf, (const float *)d_x, act, work, desc->epoch, st)) return rc;
-        const int HW = p.H * p.W, CL = p.g[p.L - 1].cout;
-        const cmma::Bnp last = cmma::bnp_of(p, act, p.L - 1);
-        PNODE_CUDA_OK(pdl::launch_pdl(cmma::act_out_kernel, dim3(dim3((HW + 31) / 32, (CL + 31) / 32, p.N)), dim3(32, 8), 0, st, (const float *)(act + p.z[p.L - 1]), last.a, last.b, CL, HW, (float *)d_k, (float *)d_out, (const float *)d_base,
-            (float)base_coef, (float)k_coef));
-        PNODE_CUDA_OK(cudaGetLastError());
-        return 0;
-    };
-    if (desc->world > 1) return launch((cudaStream_t)stream);  // the collective number changes with every call
-    gcache::Key key;
-    key.add(1).add(*desc).add(d_wbuf).add(d_x).add(d_out).add(d_base).add(base_coef).add(k_coef).add(d_k).add(d_act).add(d_work);
-    return gcache::run(key, (cudaStream_t)stream, launch);
+    cudaStream_t st = (cudaStream_t)stream;
+    uint8_t *act = (uint8_t *)d_act, *work = (uint8_t *)d_work;
+    if (int rc = cmma::forward_impl(desc, p, (const uint8_t *)d_wbuf, (const float *)d_x, act, work, desc->epoch, st)) return rc;
+    const int HW = p.H * p.W, CL = p.g[p.L - 1].cout;
+    const cmma::Bnp last = cmma::bnp_of(p, act, p.L - 1);
+    PNODE_CUDA_OK(pdl::launch_pdl(cmma::act_out_kernel, dim3(dim3((HW + 31) / 32, (CL + 31) / 32, p.N)), dim3(32, 8), 0, st, (const float *)(act + p.z[p.L - 1]), last.a, last.b, CL, HW, (float *)d_k, (float *)d_out, (const float *)d_base,
+        (float)base_coef, (float)k_coef));
+    PNODE_CUDA_OK(cudaGetLastError());
+    return 0;
 }
 
 int pnode_convmma_vjp(const pnode_convblock_desc *desc, const void *d_wbuf, const void *d_x, const void *d_w, void *d_vu,
@@ -658,7 +635,7 @@ int pnode_convmma_vjp(const pnode_convblock_desc *desc, const void *d_wbuf, cons
     Plan p;
     if (int rc = cmma::make_plan(desc, p)) return rc;
     PNODE_REQUIRE(d_wbuf && d_x && d_w && d_act && d_work, "pnode_convmma_vjp: null argument");
-    auto launch = [&](cudaStream_t st) -> int {
+    cudaStream_t st = (cudaStream_t)stream;
     const uint8_t *W = (const uint8_t *)d_wbuf;
     uint8_t *act = (uint8_t *)d_act, *work = (uint8_t *)d_work;
     float *grads = (float *)d_grads;
@@ -744,11 +721,6 @@ int pnode_convmma_vjp(const pnode_convblock_desc *desc, const void *d_wbuf, cons
         PNODE_CUDA_OK(pdl::launch_pdl(cmma::nchw_to_nhwc_kernel, dim3(dim3((C0 + 31) / 32, (HW + 31) / 32, p.N)), dim3(32, 8), 0, st, (const float *)(work + p.win), (float *)d_vu, HW, C0));
     PNODE_CUDA_OK(cudaGetLastError());
     return 0;
-    };
-    if (desc->world > 1) return launch((cudaStream_t)stream);
-    gcache::Key key;
-    key.add(2).add(*desc).add(d_wbuf).add(d_x).add(d_w).add(d_vu).add(d_grads).add(coef).add(accumulate).add(d_act).add(act_valid).add(d_work);
-    return gcache::run(key, (cudaStream_t)stream, launch);
 }
 
 }  // extern "C"

@@ -399,7 +399,6 @@ class FusedCnfRK:
         self._ckpt = None
         self._ctl_key = None
         self.device_controller = True  # -pnode_device_controller 0 falls back to one host read per attempt
-        self.device_loop = True        # -pnode_device_loop 0: stream launches in batches instead of the WHILE graph
         self.launches = 0
 
     @staticmethod
@@ -434,7 +433,7 @@ class FusedCnfRK:
         if loop.adaptive and torch.cuda.is_current_stream_capturing():
             return self._forward_captured(u0, loop, atol, rtol, save, comm)
         peer = getattr(comm, "peer", None) if comm is not None else None
-        sharded_ok = comm is None or (peer is not None and self.device_loop)  # in-kernel all-reduce of the error norm
+        sharded_ok = comm is None or peer is not None  # in-kernel all-reduce of the error norm
         if self.device_controller and loop.adaptive and sharded_ok and loop.step_list is None and \
                 (loop.span is None or len(loop.span) <= _lib.CTL_MAX_SPAN) and self.scheme.bembed is not None:
             return self._forward_device_ctl(u0, loop, atol, rtol, save, comm)
@@ -486,8 +485,7 @@ class FusedCnfRK:
         return u, sols, state
 
     # ---- adaptive run with the accept/reject decision and the next step size taken ON THE DEVICE --------------------------
-    CTL_BATCH = 8        # -pnode_device_loop 0: attempts launched between two host reads of the control block
-    CKPT_STEPS0 = 16     # checkpoint room of a fresh buffer, in steps (doubled when a solve runs out of it)
+    CKPT_STEPS0 = 16  # checkpoint room of a fresh buffer, in steps (doubled when a solve runs out of it)
 
     class _Lease:
         """A checkpoint buffer and a copy of the Hutchinson probe on loan to one solve's autograd state; they go back to the
@@ -522,8 +520,7 @@ class FusedCnfRK:
         bookkeeping (csrc/cnf_rk.cu, namespace ctl) and publishes (t, h, buffers) for the next attempt.  The whole time
         loop is ONE launch -- a CUDA graph whose WHILE node repeats the attempt kernel until the controller says stop
         (pnode_cnf_rk_solve_ctl) -- and the host reads the control block once per solve; the host TimeLoop then follows
-        the device's log (TimeLoop.follow) for the bookkeeping the caller reads.  With -pnode_device_loop 0 the attempts
-        go out as CTL_BATCH stream launches between host reads instead."""
+        the device's log (TimeLoop.follow) for the bookkeeping the caller reads."""
         sp = self.spec
         ntraj = sp.batch
         n = u0.numel()
@@ -576,19 +573,15 @@ class FusedCnfRK:
             if peer is not None:
                 _lib.check(self.lib.pnode_cnf_rk_solve_ctl_dp(*args, peer["ptrs_dev"], comm.rank, comm.world,
                                                               stream.cuda_stream))
-            elif self.device_loop:
-                _lib.check(self.lib.pnode_cnf_rk_solve_ctl(*args, stream.cuda_stream))
             else:
-                _lib.check(self.lib.pnode_cnf_rk_attempts_ctl(*args, self.CTL_BATCH, stream.cuda_stream))
-                self.launches += self.CTL_BATCH
+                _lib.check(self.lib.pnode_cnf_rk_solve_ctl(*args, stream.cuda_stream))
             self._ctl_host[:nread].copy_(self._ctl_dev[:nread], non_blocking=True)
-            stream.synchronize()  # the one host read per solve (per CTL_BATCH attempts without the device loop)
+            stream.synchronize()  # the one host read per solve
             now = c.attempts
             if peer is not None:
                 comm.collectives += int(c.epoch_next) - 1 - peer["epoch"]
                 peer["epoch"] = int(c.epoch_next) - 1
-            if self.device_loop:
-                self.launches += now - seen  # kernel nodes the graph's WHILE loop executed
+            self.launches += now - seen  # kernel nodes the graph's WHILE loop executed
             for a in range(seen, now):
                 last = a + 1 == now
                 t_next = c.t if last else c.log_t[a + 1]

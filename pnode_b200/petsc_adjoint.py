@@ -295,9 +295,7 @@ class ODEPetsc(object):
                 return None
             if self._fused is None or self._fused.scheme is not self._scheme:
                 self._fused = FusedCnfRK(self._fused_spec, self._scheme, self.tensor_dtype, self.device)
-            off = ("0", "false", "no")
-            self._fused.device_controller = Options().getString("pnode_device_controller", "1") not in off
-            self._fused.device_loop = Options().getString("pnode_device_loop", "1") not in off
+            self._fused.device_controller = Options().getString("pnode_device_controller", "1") not in ("0", "false", "no")
             self._fused.CAPTURE_ATTEMPTS = Options().getInt("pnode_capture_attempts", type(self._fused).CAPTURE_ATTEMPTS)
         return self._fused_kind, self._fused
 
@@ -356,8 +354,7 @@ class ODEPetsc(object):
                         self.tensor_dtype == torch.float64, self._max_reject)
         cb_ex, cb_im = self._active_callbacks()
         if hasattr(self._cb_ex, "layer_slices"):  # sharded runs all-reduce the wide MLP's gradient layer by layer
-            self._cb_ex.record_layer_events = self.comm is not None and getattr(self.comm, "world", 1) > 1 and \
-                Options().getString("pnode_layered_allreduce", "1") not in ("0", "false", "no")
+            self._cb_ex.record_layer_events = self.comm is not None and getattr(self.comm, "world", 1) > 1
         uf, sols = self._engine.solve(cb_ex, cb_im, self._imp, u_flat, loop, self.enable_adjoint)
         self._loop = loop
         if self._monitor:

@@ -168,7 +168,7 @@ def main():
         assert rel_err(a, b) < 2e-9, rel_err(a, b)
     if rank == 0:
         print("cnf sharded vs full batch: %d attempts, device loop on every rank: %s" %
-              (len(lb), comm.peer is not None and mine[3]._fused.device_loop), flush=True)
+              (len(lb), comm.peer is not None), flush=True)
 
     # 5. SINODE pair (BASELINE config 5 in small: circulant implicit half + wide ReLU MLP on the tensor-core evaluator), batch
     #    sharded: no exchange inside the sweep; the MLP's parameter gradient is all-reduced LAYER BY LAYER on a side stream as

@@ -142,13 +142,12 @@ def test_probe_is_sampled_like_the_reference_when_absent():
     assert ode2.path == "generic" and rel_err(out, out2) < 1e-5
 
 
-@pytest.mark.parametrize("loop_opt", [[], ["-pnode_device_loop", "0"]], ids=["while-graph", "launch-batches"])
 @pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
-def test_device_controller_follows_the_host_controller(dtype, loop_opt):
+def test_device_controller_follows_the_host_controller(dtype):
     """The accept/reject verdict and the next step size taken by the attempt kernel's last block (csrc/cnf_rk.cu, namespace
     ctl) against the host TimeLoop fed the same kernel's error norm once per attempt: same attempts, same steps, same
-    output-time copies.  The case has rejected attempts, clamped steps and three output times.  Both ways of issuing the
-    attempts: the CUDA-graph WHILE loop (one launch per solve) and batches of stream launches."""
+    output-time copies.  The case has rejected attempts, clamped steps and three output times.  The attempts run in the
+    CUDA-graph WHILE loop (one launch per solve)."""
     from pnode import petsc_adjoint
 
     B = 300
@@ -160,12 +159,11 @@ def test_device_controller_follows_the_host_controller(dtype, loop_opt):
     t = torch.tensor([0.0, 0.3, 0.35, 1.0], dtype=torch.float64)
     tol = "1e-7" if dtype == torch.float64 else "1e-4"
     argv = ["-ts_rtol", tol, "-ts_atol", tol]
-    d = _run(lambda: petsc_adjoint.ODEPetsc(), "cuda", argv + loop_opt, func, u0, t, gout, "dopri5", 0.5)
+    d = _run(lambda: petsc_adjoint.ODEPetsc(), "cuda", argv, func, u0, t, gout, "dopri5", 0.5)
     h = _run(lambda: petsc_adjoint.ODEPetsc(), "cuda", argv + ["-pnode_device_controller", "0"], func, u0, t, gout, "dopri5",
              0.5)
     assert d[3].path == h[3].path == "fused-cnf-rk"
     assert d[3]._fused.device_controller and not h[3]._fused.device_controller
-    assert d[3]._fused.device_loop == (not loop_opt)
     la, lb = d[3]._loop.attempts, h[3]._loop.attempts
     if dtype == torch.float64:
         assert any(not a[2] for a in la), "case must contain a rejected attempt"
@@ -179,8 +177,7 @@ def test_device_controller_follows_the_host_controller(dtype, loop_opt):
     _compare(d, h, 1e-11 if dtype == torch.float64 else 1e-4)
 
 
-@pytest.mark.parametrize("loop_opt", [[], ["-pnode_device_loop", "0"]], ids=["while-graph", "launch-batches"])
-def test_device_controller_many_steps_and_single_end_time(loop_opt):
+def test_device_controller_many_steps_and_single_end_time():
     """More accepted steps than the checkpoint buffer starts with (the device loop stops with done = 4, the host doubles
     the buffer and the loop goes on); one-element t (no span); two solves in a row on the same object (buffers and the
     cached loop graph are reused).  Compared with the host-controlled run of the same kernels (at this tolerance the
@@ -193,16 +190,16 @@ def test_device_controller_many_steps_and_single_end_time(loop_opt):
     u0, gout = _inputs(B, 6, 1, torch.float64)
     t = torch.tensor([1.0], dtype=torch.float64)
     argv = ["-ts_rtol", "1e-10", "-ts_atol", "1e-10"]
-    room, batch = FusedCnfRK.CKPT_STEPS0, FusedCnfRK.CTL_BATCH
-    FusedCnfRK.CKPT_STEPS0, FusedCnfRK.CTL_BATCH = 2, 3
+    room = FusedCnfRK.CKPT_STEPS0
+    FusedCnfRK.CKPT_STEPS0 = 2
     try:
-        d = _run(lambda: petsc_adjoint.ODEPetsc(), "cuda", argv + loop_opt, func, u0, t, gout, "dopri5", 0.01)
+        d = _run(lambda: petsc_adjoint.ODEPetsc(), "cuda", argv, func, u0, t, gout, "dopri5", 0.01)
         ode = d[3]
         y0 = u0.to("cuda").clone().requires_grad_(True)
         again = ode.odeint_adjoint(y0, t.to("cuda"))  # same object: pooled checkpoint buffer, cached graph
         lam_again, = torch.autograd.grad((again * gout.to("cuda")).sum(), [y0])
     finally:
-        FusedCnfRK.CKPT_STEPS0, FusedCnfRK.CTL_BATCH = room, batch
+        FusedCnfRK.CKPT_STEPS0 = room
     h = _run(lambda: petsc_adjoint.ODEPetsc(), "cuda", argv + ["-pnode_device_controller", "0"], func, u0, t, gout, "dopri5",
              0.01)
     assert d[3].path == "fused-cnf-rk" and d[3]._fused.device_controller and not h[3]._fused.device_controller
