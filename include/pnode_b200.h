@@ -146,8 +146,11 @@ typedef struct pnode_step {
  *   d_u0     [ntraj, dim]                 initial states (C-order flatten of the caller's tensor, petsc_adjoint.py:596)
  *   d_sched  DEVICE [nsteps] pnode_step   schedule
  *   d_sol    [nout, ntraj, dim]           span solutions (slots named by out_slot; others untouched)
- *   d_ckpt   [nsteps, s, dim, ntraj]      stage values Y_i, or NULL when no adjoint will follow
+ *   d_ckpt   [nsteps, s, rows, ntraj]     stage checkpoints, rows = pnode_mlp_rk_ckpt_rows(): the stage value Y_i in rows
+ *                                         0..dim-1, for some shapes followed by the stage Jacobian df/dy(Y_i) (dim x dim,
+ *                                         row-major) that the adjoint sweep uses; NULL when no adjoint will follow
  */
+int pnode_mlp_rk_ckpt_rows(const pnode_mlp_desc *mlp, const pnode_rk_tableau *tab);
 int pnode_mlp_rk_forward(const pnode_mlp_desc *mlp, const pnode_rk_tableau *tab, const void *d_u0, int64_t ntraj,
                          const pnode_step *d_sched, int nsteps, void *d_sol, void *d_ckpt, void *stream);
 
@@ -156,6 +159,7 @@ int pnode_mlp_rk_forward(const pnode_mlp_desc *mlp, const pnode_rk_tableau *tab,
  * RHSJacShell.multTranspose / RHSJacPShell.multTranspose callbacks fused in; lambda += grad_out[in_slot] after the
  * adjoint of a step that starts at an output point (the reference's forcing, petsc_adjoint.py:938).
  *   d_gout   [nout, ntraj, dim]   dL/d(solution slots)
+ *   d_ckpt   the stage checkpoints pnode_mlp_rk_forward wrote ([nsteps, s, pnode_mlp_rk_ckpt_rows(), ntraj])
  *   d_lambda [ntraj, dim]         out: dL/du0
  *   d_mu     [np]                 out: dL/dparams, order W1,b1,W2,b2 (func.parameters() order, petsc_adjoint.py:618-620)
  *   d_work   scratch of pnode_mlp_rk_adjoint_work_bytes() bytes, zero-initialised once by the caller (per-block partial
@@ -168,8 +172,8 @@ int pnode_mlp_rk_adjoint(const pnode_mlp_desc *mlp, const pnode_rk_tableau *tab,
 
 /* Bounded checkpoint storage for the fused sweeps: [PETSc] -ts_trajectory_solution_only 1 (TSTrajectory "memory" keeping
  * the step solutions only, SURVEY.md A.7; the reference reaches it through ts.setFromOptions(), petsc_adjoint.py:775).
- * The forward sweep keeps u_n per step -- d_usteps [nsteps, dim, ntraj], 1/s of the stage checkpoints -- and the adjoint
- * sweep recomputes the s stage values of a step from u_n with the forward sweep's own arithmetic before it runs the
+ * The forward sweep keeps u_n per step -- d_usteps [nsteps, dim, ntraj], at most 1/s of the stage checkpoints -- and the adjoint
+ * sweep recomputes the s stage values (and stage Jacobians) of a step from u_n with the forward sweep's own arithmetic before it runs the
  * step's adjoint stages (same results as the stage-checkpoint sweeps, bit for bit).  d_peer_bufs NULL / world 1: single
  * GPU; otherwise as pnode_mlp_rk_adjoint_dp. */
 int pnode_mlp_rk_forward_so(const pnode_mlp_desc *mlp, const pnode_rk_tableau *tab, const void *d_u0, int64_t ntraj,

@@ -99,6 +99,7 @@ _SIGNATURES = {
     "pnode_lincomb_seg": (C.c_int, [_vp, _vp, _d, _vp, _vp, _i, _i, _i64, _i64, _i, _vp]),
     "pnode_mlp_rk_supported": (C.c_int, [_i, _i, _i, _i, _i]),
     "pnode_mlp_rk_forward": (C.c_int, [C.POINTER(MlpDesc), C.POINTER(RKTableau), _vp, _i64, _vp, _i, _vp, _vp, _vp]),
+    "pnode_mlp_rk_ckpt_rows": (C.c_int, [C.POINTER(MlpDesc), C.POINTER(RKTableau)]),
     "pnode_mlp_rk_adjoint_work_bytes": (_i64, [C.POINTER(MlpDesc)]),
     "pnode_mlp_rk_adjoint": (C.c_int, [C.POINTER(MlpDesc), C.POINTER(RKTableau), _i64, _vp, _i, _i, _vp, _vp, _vp, _vp,
                                        _vp, _vp]),

@@ -190,12 +190,13 @@ class FusedMlpRK:
             sol[0].copy_(u0)
         ckpt = None
         so = bool(self.solution_only and save)
+        desc = self._desc()
         if save:
-            shape = (max(nsteps, 1), sp.dim, ntraj) if so else (max(nsteps, 1), self.scheme.s, sp.dim, ntraj)
+            rows = int(self.lib.pnode_mlp_rk_ckpt_rows(C.byref(desc), C.byref(self.tab)))
+            shape = (max(nsteps, 1), sp.dim, ntraj) if so else (max(nsteps, 1), self.scheme.s, rows, ntraj)
             ckpt = torch.empty(shape, dtype=self.dtype, device=self.device)
         if nsteps == 0:
             sol[-1].copy_(u0)
-        desc = self._desc()
         fwd = self.lib.pnode_mlp_rk_forward_so if so else self.lib.pnode_mlp_rk_forward
         _lib.check(fwd(C.byref(desc), C.byref(self.tab), u0.data_ptr(), ntraj, sched.data_ptr(), nsteps, sol.data_ptr(),
                        None if ckpt is None else ckpt.data_ptr(), _stream()))
