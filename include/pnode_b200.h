@@ -506,12 +506,15 @@ int pnode_dmlp_vjp_ev(const pnode_dmlp_desc *desc, const void *d_wslices, const 
 
 /* ----------------------------------------------------------------------------------------------------------------
  * FFJORD right-hand side with an ODEnet of any depth (csrc/cnf_net.cu): L ConcatSquashLinear layers with Softplus(beta=1,
- * threshold=20) between them, Hutchinson trace with the probe d_e, state cat(z.view(-1), logp.view(-1)) of B samples.
+ * threshold=20) between them, state cat(z.view(-1), logp.view(-1)) of B samples.  The trace is the Hutchinson estimate
+ * e^T J e with the probe d_e (trace = 0, divergence_approx) or the exact trace tr J (trace = 1, divergence_bf; d_e is not
+ * read), formed as the forward tangents of one chain (e) or of D chains (the unit vectors).
  * Replaces ODEfunc.forward (ffjord-pnode/lib/layers/odefunc.py:53-57, 345-385; ConcatSquashLinear, diffeq_layers/basic.py:
  * 76-86) in evalRHSFunction, and the second-order autograd of RHSJacShell.multTranspose + RHSJacPShell.multTranspose
  * (pnode/petsc_adjoint.py:52-82, 341-363) in every adjoint stage.  Every product runs on the tensor cores through the
- * sliced operands above (fp64: int8 slices, I8X when 2B or a width exceeds PNODE_I8_MAX_K; fp32: 3xTF32), with the value
- * and tangent chains stacked as 2B rows.
+ * sliced operands above (fp64: int8 slices, I8X when (1 + chains) B or a width exceeds PNODE_I8_MAX_K; fp32: 3xTF32), with
+ * the value and tangent chains stacked as (1 + chains) B rows (2B for the Hutchinson trace, (D + 1) B for the exact one),
+ * which must be within one product's reduction length (PNODE_I8X_MAX_K in fp64, 65536 in fp32).
  *   prepare : slice every weight matrix in both orientations (once per solve: parameters are borrowed)
  *   forward : d_out[B*(D+1)] = F(t, d_u); with d_act != NULL the evaluation keeps what the adjoint stage at the same point
  *             needs (column-sliced layer inputs, pre-activations, gates)
@@ -529,7 +532,8 @@ typedef struct pnode_cnfnet_desc {
     const void *d_gate_bias[PNODE_DMLP_MAX_LAYERS];   /* _hyper_gate.bias [dims[l+1]] */
     int64_t mu_w_off[PNODE_DMLP_MAX_LAYERS], mu_b_off[PNODE_DMLP_MAX_LAYERS], mu_hbw_off[PNODE_DMLP_MAX_LAYERS],
         mu_hgw_off[PNODE_DMLP_MAX_LAYERS], mu_hgb_off[PNODE_DMLP_MAX_LAYERS];
-    const void *d_e;                              /* [B][D] Hutchinson probe */
+    const void *d_e;                              /* [B][D] Hutchinson probe (read when trace = 0) */
+    int32_t trace;                                /* 0: Hutchinson e^T J e, 1: exact tr J */
 } pnode_cnfnet_desc;
 int64_t pnode_cnfnet_weight_bytes(const pnode_cnfnet_desc *desc);   /* -1: unsupported (pnode_last_error) */
 int64_t pnode_cnfnet_act_bytes(const pnode_cnfnet_desc *desc);

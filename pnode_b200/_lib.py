@@ -68,7 +68,7 @@ class CnfNetDesc(C.Structure):
                [(n, C.c_void_p * DMLP_MAX_LAYERS) for n in ("d_weight", "d_bias", "d_hyper_bias", "d_gate_weight",
                                                             "d_gate_bias")] + \
                [(n, C.c_int64 * DMLP_MAX_LAYERS) for n in ("mu_w_off", "mu_b_off", "mu_hbw_off", "mu_hgw_off",
-                                                          "mu_hgb_off")] + [("d_e", C.c_void_p)]
+                                                          "mu_hgb_off")] + [("d_e", C.c_void_p), ("trace", C.c_int32)]
 
 
 class ConvLayer(C.Structure):

@@ -1,10 +1,12 @@
 """FFJORD right-hand sides of any depth on the tensor cores: an evaluator plugged into the generic stage loop.
 
   * CnfNetCallbacks -- F(t, y) of FlattenFunc(ODEfunc(ODEnet)) with L ConcatSquashLinear layers, Softplus between them and
-                       the Hutchinson trace (ffjord-pnode/lib/layers/odefunc.py:53-57,345-385, cnf.py:72-80): one C call per
-                       evaluation and one per adjoint stage into csrc/cnf_net.cu.  The trace is the forward tangent of the
-                       probe, so neither the forward nor the adjoint needs autograd (the reference differentiates the
-                       autograd trace a second time in every adjoint stage, petsc_adjoint.py:52-82,341-363).  Weight gradients
+                       the Hutchinson trace (divergence_approx) or the exact trace (divergence_bf)
+                       (ffjord-pnode/lib/layers/odefunc.py:21-57,345-385, cnf.py:72-80): one C call per evaluation and one
+                       per adjoint stage into csrc/cnf_net.cu.  The trace is the forward tangent of the probe (or of the D
+                       unit vectors, for the exact trace), so neither the forward nor the adjoint needs autograd (the
+                       reference differentiates the autograd trace a second time in every adjoint stage,
+                       petsc_adjoint.py:52-82,341-363; its exact trace takes D autograd calls per evaluation).  Weight gradients
                        are accumulated straight into mu; the forward keeps an activation set per stage evaluation so the
                        adjoint does not re-evaluate.
 The module is recognised by fused.recognise_cnf (structure + numerical probe through the user's module)."""
@@ -22,6 +24,7 @@ from .fused import hutchinson_probe
 def _desc_for(spec, dtype):
     d = _lib.CnfNetDesc()
     d.nlayers, d.dtype, d.batch, d.t_f32 = len(spec.layers), dtype_code(dtype), spec.batch, spec.t_via_f32
+    d.trace = 1 if spec.trace == "exact" else 0
     for l, n in enumerate(spec.dims):
         d.dims[l] = n
     return d
@@ -30,7 +33,8 @@ def _desc_for(spec, dtype):
 class CnfNetCallbacks(Callbacks):
     @staticmethod
     def supported(spec, dtype):
-        """Depth and every reduction length (widths and 2 x batch) within what one sliced product takes."""
+        """Depth and every reduction length (widths and (1 + chains) x batch: 2B for the Hutchinson trace, (D + 1) B for
+        the exact one) within what one sliced product takes."""
         if len(spec.layers) > _lib.DMLP_MAX_LAYERS:
             return False
         d = _desc_for(spec, dtype)
@@ -86,7 +90,9 @@ class CnfNetCallbacks(Callbacks):
             self.launches += len(self.spec.layers)
 
     def _probe(self):
-        """FFJORD draws a fresh probe per solve (before_odeint): the descriptor follows the module's current one."""
+        """FFJORD draws a fresh probe per solve (before_odeint): the descriptor follows the module's current one.  The
+        module draws it before it picks a divergence, so it is drawn for the exact trace too (which does not read it): the
+        caller's RNG stream and `_e` end up as the module leaves them."""
         sp = self.spec
         e = hutchinson_probe(sp.odefunc, sp.batch, sp.dim, self.dtype, self.device)
         self._desc.d_e = e.data_ptr()

@@ -246,7 +246,8 @@ class FusedMlpRK:
 
 class CnfSpec:
     """A recognised FFJORD right-hand side: ODEfunc `odefunc` over L ConcatSquashLinear `layers` (widths `dims`, dims[0] =
-    dims[L] = D) and a batch of B samples.  `l1`, `l2`, `hidden` describe the two-layer shape of the fused sweeps."""
+    dims[L] = D) and a batch of B samples.  `l1`, `l2`, `hidden` describe the two-layer shape of the fused sweeps.  `trace`
+    is what the module's divergence computes: "hutchinson" (e^T J e, divergence_approx) or "exact" (tr J, divergence_bf)."""
 
     def __init__(self, odefunc, layers, batch, dim):
         self.odefunc, self.layers = odefunc, list(layers)
@@ -254,6 +255,7 @@ class CnfSpec:
         self.dims = [dim] + [m._layer.out_features for m in self.layers]
         self.l1, self.l2, self.hidden = self.layers[0], self.layers[-1], self.dims[1]
         self.t_via_f32 = 1
+        self.trace = "hutchinson"
 
     @staticmethod
     def layer_params(m):
@@ -266,8 +268,9 @@ class CnfSpec:
         return out
 
 
-# odefunc -> {(id(diffeq), dims, dtype, device): (weakref to diffeq, t_via_f32)} once the numerical probe has passed.  Weak in
-# both modules: a verdict must not pass to a new module that CPython places at the address of a freed one.
+# odefunc -> {(id(diffeq), dims, dtype, device, training): (weakref to diffeq, t_via_f32, trace)} once the numerical probe has
+# passed.  Weak in both modules: a verdict must not pass to a new module that CPython places at the address of a freed one.
+# The training flag is part of the key because FFJORD's ODEfunc switches to the exact trace in eval mode for 2-D states.
 _CNF_RECOGNISED = weakref.WeakKeyDictionary()
 
 
@@ -278,10 +281,13 @@ def _is_concatsquash(m):
             and m._hyper_gate.in_features == 1)
 
 
-def cnf_closed_form(layers, z, e, t):
+def cnf_closed_form(layers, z, e, t, exact=False):
     """(f, div) of the ConcatSquash network at time tensor t, the Hutchinson trace div = e^T (df/dz) e formed as the forward
-    tangent of e -- the formula csrc/cnf_net.cu evaluates (and, for two layers, csrc/cnf_rk.cu)."""
-    x, v = z, e
+    tangent of e -- the formula csrc/cnf_net.cu evaluates (and, for two layers, csrc/cnf_rk.cu).  With exact=True, div is
+    the exact trace tr(df/dz), the sum of the diagonals of the forward tangents of the D unit vectors (e is not read)."""
+    B, D = z.shape
+    x = z
+    v = torch.eye(D, dtype=z.dtype, device=z.device)[:, None, :].expand(D, B, D) if exact else e[None]
     for l, m in enumerate(layers):
         gam = torch.sigmoid(m._hyper_gate(t.view(1, 1)))
         a = m._layer(x) * gam + m._hyper_bias(t.view(1, 1))
@@ -289,7 +295,9 @@ def cnf_closed_form(layers, z, e, t):
         if l < len(layers) - 1:
             x = torch.nn.functional.softplus(a)
             v = torch.where(a > 20, torch.ones_like(a), torch.sigmoid(a)) * u
-    return a, (e * u).sum(1)
+    if exact:
+        return a, torch.diagonal(u, dim1=0, dim2=2).sum(1)
+    return a, (e * u[0]).sum(1)
 
 
 def hutchinson_probe(bf, batch, dim, dtype, device):
@@ -308,9 +316,11 @@ def hutchinson_probe(bf, batch, dim, dtype, device):
 
 def recognise_cnf(func, u_meta):
     """Match the object graph cnf.py:72-80 builds -- FlattenFunc(base_func=ODEfunc(diffeq=ODEnet(L >= 1 ConcatSquashLinear
-    layers with Softplus between them), divergence_approx, residual=False), y0=(z [B,D], logp [B,1])) -- by duck typing,
-    then confirm with a numerical probe that func(t, y) equals cnf_closed_form (once per diffeq module).  Which runner
-    evaluates it (the two-layer fused sweeps or the evaluator of any depth) is decided where the runner is chosen."""
+    layers with Softplus between them), divergence_approx or divergence_bf, residual=False), y0=(z [B,D], logp [B,1])) -- by
+    duck typing, then confirm with a numerical probe that func(t, y) equals cnf_closed_form (once per diffeq module and
+    training flag).  The probe, not the divergence_fn attribute, decides the trace kind: FFJORD's ODEfunc takes the exact
+    trace in eval mode for 2-D states whatever its divergence_fn.  Which runner evaluates it (the two-layer fused sweeps
+    for the Hutchinson trace, or the evaluator of any depth) is decided where the runner is chosen."""
     bf, y0 = getattr(func, "base_func", None), getattr(func, "y0", None)
     if bf is None or not isinstance(y0, (tuple, list)) or len(y0) != 2 or not u_meta.is_cuda:
         return None
@@ -327,7 +337,7 @@ def recognise_cnf(func, u_meta):
         return None
     if any(a.beta != 1 or a.threshold != 20 for a in acts) or getattr(bf, "residual", False):
         return None
-    if getattr(getattr(bf, "divergence_fn", None), "__name__", "") != "divergence_approx":
+    if getattr(getattr(bf, "divergence_fn", None), "__name__", "") not in ("divergence_approx", "divergence_bf"):
         return None
     B, D = z0.shape
     layers = list(layers)
@@ -342,7 +352,7 @@ def recognise_cnf(func, u_meta):
     if any(p.dtype != u_meta.dtype or p.device != u_meta.device or not p.is_contiguous() for p in want):
         return None
     seen = _CNF_RECOGNISED.setdefault(bf, {})
-    key = (id(net), tuple(spec.dims), u_meta.dtype, str(u_meta.device))
+    key = (id(net), tuple(spec.dims), u_meta.dtype, str(u_meta.device), bool(bf.training))
     if key not in seen or seen[key][0]() is not net:
         # probe through the user's module itself (FlattenFunc -> ODEfunc -> ODEnet), on a small batch, at times that are
         # not representable in float32 so that the module's handling of `t` is observable
@@ -358,17 +368,22 @@ def recognise_cnf(func, u_meta):
                 bf._e = e
                 tol = 2e-4 if u_meta.dtype == torch.float32 else 1e-11
                 verdict = None
-                for via_f32 in (1, 0):
-                    ok = True
-                    for tval in (0.3, 0.9):
-                        got = type(func)(bf, (z, torch.zeros(nb, 1).to(u_meta)))(tval, torch.cat((z.reshape(-1),
-                                                                                  torch.zeros(nb).to(u_meta))))
-                        t = torch.tensor(tval).to(u_meta) if via_f32 else torch.tensor(tval, dtype=torch.float64).to(u_meta)
-                        f, div = cnf_closed_form(layers, z, e, t)
-                        ref = torch.cat((f.reshape(-1), -div))
-                        ok = ok and got.shape == ref.shape and torch.allclose(got.detach(), ref, rtol=tol, atol=tol)
-                    if ok:
-                        verdict = via_f32
+                got = [type(func)(bf, (z, torch.zeros(nb, 1).to(u_meta)))(tval, torch.cat((z.reshape(-1),
+                                                                           torch.zeros(nb).to(u_meta)))).detach()
+                       for tval in (0.3, 0.9)]
+                for trace in ("hutchinson", "exact"):
+                    for via_f32 in (1, 0):
+                        ok = True
+                        for tval, g_t in zip((0.3, 0.9), got):
+                            t = torch.tensor(tval).to(u_meta) if via_f32 else \
+                                torch.tensor(tval, dtype=torch.float64).to(u_meta)
+                            f, div = cnf_closed_form(layers, z, e, t, exact=trace == "exact")
+                            ref = torch.cat((f.reshape(-1), -div))
+                            ok = ok and g_t.shape == ref.shape and torch.allclose(g_t, ref, rtol=tol, atol=tol)
+                        if ok:
+                            verdict = (via_f32, trace)
+                            break
+                    if verdict is not None:
                         break
         except Exception:
             verdict = None
@@ -378,8 +393,8 @@ def recognise_cnf(func, u_meta):
                 bf._num_evals.copy_(nevals)  # the probe is not an evaluation of the user's solve
         if verdict is None:
             return None
-        seen[key] = (weakref.ref(net), verdict)
-    spec.t_via_f32 = seen[key][1]
+        seen[key] = (weakref.ref(net),) + verdict
+    spec.t_via_f32, spec.trace = seen[key][1], seen[key][2]
     return spec
 
 
@@ -404,8 +419,10 @@ class FusedCnfRK:
 
     @staticmethod
     def supported(spec, scheme, dtype):
-        return len(spec.layers) == 2 and bool(_lib.load().pnode_cnf_rk_supported(spec.dim, spec.hidden, dtype_code(dtype),
-                                                                                  scheme.s))
+        """The sweeps carry the Hutchinson trace only: an exact-trace module takes the evaluator of any depth."""
+        if spec.trace != "hutchinson" or len(spec.layers) != 2:
+            return False
+        return bool(_lib.load().pnode_cnf_rk_supported(spec.dim, spec.hidden, dtype_code(dtype), scheme.s))
 
     def _desc(self):
         sp = self.spec
